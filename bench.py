@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on the host cores
+    python bench.py --gpus 1 ... --dump-outputs DIR          # also write the last timed step's frames to DIR/*.npy
 
 A step = one pass of the hot path (envelope -> slicer -> Manchester/Miller -> frames) over one synthetic
 ISO 14443A capture that is already resident in HBM.  N=1 workload: BASELINE.json configs[2], 1e10 samples at
@@ -113,6 +114,32 @@ def same_frames(ra, rb):
         return False
     return bool(np.array_equal(fa["pos"], fb["pos"]) and np.array_equal(fa["type"], fb["type"]) and
                 np.array_equal(fa["nbits"], fb["nbits"]) and np.array_equal(a0, b0) and np.array_equal(a1, b1))
+
+
+DUMP_FRAMES = 1 << 21  # --dump-outputs: frame records written whole up to this many, else a seeded sample of this many
+DUMP_BITS = 1 << 21    # frame bits of each direction, likewise
+
+
+def sample_index(n, k, seed):
+    """Sorted indices of a fixed, seeded sample of k of n items (all n when n <= k)."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, frames):
+    """What a caller of the timed decode receives, as out_dir/<name>.npy: the frame records (closing position in float64, type
+    and length in float32) and the tag -> reader and reader -> tag frame bits (float32), each capped as above: at most 48 MiB.
+    frames: (records, tag bits, reader bits) as view_frames returns them.  Two builds that decode alike write identical files."""
+    fr, b0, b1 = frames
+    i = sample_index(len(fr), DUMP_FRAMES, 1)
+    out = {"frame_pos": fr["pos"][i].astype(np.float64), "frame_type": fr["type"][i].astype(np.float32),
+           "frame_nbits": fr["nbits"][i].astype(np.float32),
+           "bits_tag": b0[sample_index(len(b0), DUMP_BITS, 2)].astype(np.float32),
+           "bits_reader": b1[sample_index(len(b1), DUMP_BITS, 3)].astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def oracle_windows(x, frames, params, k, wlen=6_000_000):
@@ -560,13 +587,19 @@ def main():
                          "blocking waits were no faster)")
     ap.add_argument("--fade", type=float, default=0.05, help="channel: slow amplitude fade depth (experiments)")
     ap.add_argument("--tag-high", type=float, default=1.07, help="channel: tag load-modulation amplitude ratio (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the frames of the last one to DIR/<name>.npy "
+                                                          "(records and a seeded sample of the frame bits; inputs are seeded)")
     args = ap.parse_args()
-    quiet_stdout()
-    globals()["RATE"] = args.rate
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps: at least one timed step")
+    if args.dump_outputs and (args.impl != "b200" or args.batch > 0 or world > 1):
+        ap.error("--dump-outputs: the decode of one capture on one GPU only (no --batch, --impl reference or several ranks)")
+    quiet_stdout()
+    globals()["RATE"] = args.rate
     import torch
     import torch.distributed as dist
 
@@ -650,13 +683,14 @@ def main():
         room = shm_room()
         shared = sharding.SharedFrameIndex(s, want_recs if room > 4 * world * want_recs * 8 else 0, dist)
 
-    def step():
+    def step(keep=False):
         if world == 1:
             s.reset()
             s.push_all(x)
             fr, _, _ = s.view_frames()  # records and frame bits in host memory (zero-copy view of the library's buffers)
             nfr = len(fr)
-            s.release_frames()
+            if not keep:  # (kept: dumped and released once the clock has stopped)
+                s.release_frames()
             return nfr
         res = sharding.decode_time_sharded(s, lambda a, b: x[a - base: b - base], total, L, _cabi.State, dist=dist,
                                            device="cuda", halo_windows=args.halo_windows, flat="view")
@@ -691,13 +725,16 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.perf_counter()
     ev0.record()
-    for _ in range(args.steps):
-        frames = step()
+    for i in range(args.steps):
+        frames = step(keep=bool(args.dump_outputs) and i == args.steps - 1)
     ev1.record()
     barrier()
     wall = time.perf_counter() - t0
     st = s.stats()
     clocks = sampler.stop(t_load, t0, t0 + wall) if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, s.view_frames())
+        s.release_frames()
     # device time of the step on the library's own stream (CUDA events inside the library bracket every slab)
     dev_ms = st["kernel_ms"] / args.steps
     wall_ms = wall * 1e3 / args.steps

@@ -44,15 +44,18 @@ def test_transition_buffer_overflow_is_retried():
     assert got["stream"].stats()["overflow_retries"] > 0
 
 
-def test_seam_mismatches_are_found_and_repaired():
-    """Segments of four tiles with a halo of one: speculative starts inside frames do not converge in time, the seam check
-    finds them and the repair restores the exact stream."""
+@pytest.mark.parametrize("av_window,seg_len,halo", [(2000, 4096, 1024), (1000, 1024, 256), (1002, 1024, 256)])
+def test_seam_mismatches_are_found_and_repaired(av_window, seg_len, halo):
+    """Short segments with a short halo: speculative starts inside frames do not converge in time, the seam check finds
+    them and the repair restores the exact stream.  av_window 2000: the streaming kernel (class bitmap); 1000 and 1002:
+    the first-generation kernel (transition lists, tiles of 256 samples: segments of four tiles with a halo of one), with a
+    window that is a multiple of 4 and one that is not."""
     rate = 2e6
     frames = synth.load_sessions()["classic1k"]
-    pcm = synth.capture(frames, rate, 77, channel=synth.Channel(pause=0.03, tag_high=1.07, fade=0.06), av_window=2000)
+    pcm = synth.capture(frames, rate, 77, channel=synth.Channel(pause=0.03, tag_high=1.07, fade=0.06), av_window=av_window)
     x = synth.envelope(synth.pcm_to_float(pcm))
-    want = oracle.decode_capture(x, rate, hi_val=1.09)
-    got = gpu_decode(x, rate, hi_val=1.09, tuning=dict(seg_len=4096, halo=1024))
+    want = oracle.decode_capture(x, rate, hi_val=1.09, av_window=av_window)
+    got = gpu_decode(x, rate, hi_val=1.09, av_window=av_window, tuning=dict(seg_len=seg_len, halo=halo))
     check_against_oracle(got, want)
     st = got["stream"].stats()
     assert st["segments"] > 20 and st["seam_mismatches"] > 0

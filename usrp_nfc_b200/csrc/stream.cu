@@ -239,7 +239,7 @@ struct Stream {
     int force_serial = 0;
 
     // device scratch
-    DevBuf params_d, tab_d, staging, works_d, states_d, trans_seg, seg_counts, seg_offsets, seg_status,
+    DevBuf params_d, tab_d, staging, works_d, states_d, trans_seg, seg_counts, seg_status,
         seam_ptrs, mismatch_d, run_counts, run_offsets, scan_scr, maps_d, prefix_d, cnts_d, cprefix_d,
         line_scr, serial_ring, start_d, ckpt_d, redo_states, redo_trans,
         redo_counts, pieces_d, bitmap_d, ex_counts, ex_offsets, ex_scr, summ_d;
@@ -348,9 +348,15 @@ struct Stream {
     DevBuf batch_states, batch_stage;
     int finish_warmup();
     int process_slab(const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b, int64_t slicer_end);
-    int run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b, bool serial, uint32_t *R_out,
-                   bool *fell_back);
-    int run_slicer_bm(const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b, bool *fell_back);
+    // the streaming kernel writes the class bitmap; the first-generation kernel (windows below 1024 samples or not a
+    // multiple of 4) and the sequential kernel write transition lists
+    enum class Slicer { streaming, first_gen, sequential };
+    int run_slicer(Slicer kind, const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b,
+                   uint32_t *R_out, bool *fell_back);
+    int launch_streaming(const SegWork *d_works, int n_works);
+    void add_kernel_time();
+    int compare_states(const std::vector<const SlicerHdr *> &truth, const std::vector<const SlicerHdr *> &assumed, int n,
+                       std::vector<int> &mism);
     // the class bitmap holds stream positions [bm_lo, bm_hi) (chunk 0 at bm_origin): the streaming slicer may run ahead of the
     // slab that is being turned into events
     int64_t bm_lo = 0, bm_hi = 0, bm_origin = 0;
@@ -473,7 +479,7 @@ int Stream::init(const nfc_params *p) {
 }
 
 void Stream::destroy() {
-    DevBuf *all[] = {&batch_states, &batch_stage, &params_d, &tab_d, &staging, &works_d, &states_d, &trans_seg, &trans_dense[0], &trans_dense[1], &seg_counts, &seg_offsets,
+    DevBuf *all[] = {&batch_states, &batch_stage, &params_d, &tab_d, &staging, &works_d, &states_d, &trans_seg, &trans_dense[0], &trans_dense[1], &seg_counts,
                      &seg_status, &seam_ptrs, &mismatch_d, &run_counts, &run_offsets, &scan_scr, &maps_d,
                      &prefix_d, &cnts_d, &cprefix_d, &line_scr, &ctx_d, &events_d[0], &events_d[1], &sym_d[0], &sym_d[1], &bits0_d[0],
                      &bits0_d[1], &bits1_d[0], &bits1_d[1], &em_d[0], &em_d[1], &fx_d[0], &fx_d[1],
@@ -784,22 +790,14 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
         w.bm_pos0 = 0;
     }
     NFC_CUDA_CHECK(cudaMemcpyAsync(works_d.p, works.data(), sizeof(SegWork) * (size_t)n_cap, cudaMemcpyHostToDevice, cs));
-    NFC_CUDA_CHECK(cudaEventRecord(ev_k0, cs));
-    if (launch_slicer_streaming(works_d.as<SegWork>(), (int)n_cap, params_d.as<SlicerParams>(), L, sp.input_kind, cs)) return -1;
-    NFC_CUDA_CHECK(cudaEventRecord(ev_k1, cs));
+    if (launch_streaming(works_d.as<SegWork>(), (int)n_cap)) return -1;
     stats.launches++;
     stats.slicer_launches++;
     stats.segments += n_cap;
     std::vector<int32_t> status((size_t)n_cap);
     NFC_CUDA_CHECK(cudaMemcpyAsync(status.data(), seg_status.p, sizeof(int32_t) * (size_t)n_cap, cudaMemcpyDeviceToHost, cs));
     NFC_CUDA_CHECK(sync_cs());
-    {
-        float ms = 0;
-        if (cudaEventElapsedTime(&ms, ev_k0, ev_k1) == cudaSuccess) {
-            stats.slicer_kernel_ms += ms;
-            stats.slicer_kernel_launches++;
-        }
-    }
+    add_kernel_time();
     for (int64_t c = 0; c < n_cap; c++)
         if (status[(size_t)c] & (SEG_INEXACT | SEG_NOT_SANE)) {
             set_error("push_batch: capture %lld is outside the exactly-summable regime: decode the captures one by one", (long long)c);
@@ -837,10 +835,79 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
     return rc ? rc : n_cap;
 }
 
-// Runs the slicer over [a, b) and leaves the dense ordered transitions in trans_dense (count in *R_out) and the
-// true final state in `state`.
-int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b, bool serial,
+// Launches the streaming slicer kernel between ev_k0 and ev_k1; add_kernel_time() counts its time once the stream has been
+// synchronised.
+int Stream::launch_streaming(const SegWork *d_works, int n_works) {
+    NFC_CUDA_CHECK(cudaEventRecord(ev_k0, cs));
+    if (launch_slicer_streaming(d_works, n_works, params_d.as<SlicerParams>(), sp.L, sp.input_kind, cs)) return -1;
+    NFC_CUDA_CHECK(cudaEventRecord(ev_k1, cs));
+    return 0;
+}
+
+void Stream::add_kernel_time() {
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, ev_k0, ev_k1) == cudaSuccess) {
+        stats.slicer_kernel_ms += ms;
+        stats.slicer_kernel_launches++;
+    }
+}
+
+// Queues the bit-for-bit comparison of the states truth[q] and assumed[q], q < n (a pair with a nullptr is skipped);
+// mism[q] is set once the stream has been synchronised.  seam_ptrs has room for truth.size() entries of each kind.
+int Stream::compare_states(const std::vector<const SlicerHdr *> &truth, const std::vector<const SlicerHdr *> &assumed, int n,
+                           std::vector<int> &mism) {
+    const size_t room = truth.size();
+    char *base = seam_ptrs.as<char>();
+    NFC_CUDA_CHECK(cudaMemcpyAsync(base, truth.data(), sizeof(void *) * (size_t)n, cudaMemcpyHostToDevice, cs));
+    NFC_CUDA_CHECK(cudaMemcpyAsync(base + sizeof(void *) * room, assumed.data(), sizeof(void *) * (size_t)n, cudaMemcpyHostToDevice, cs));
+    NFC_CUDA_CHECK(cudaMemsetAsync(base + 2 * sizeof(void *) * room, 0, sizeof(int) * (size_t)n, cs));  // parameter set 0
+    NFC_CUDA_CHECK(cudaMemsetAsync(mismatch_d.p, 0, sizeof(int) * (size_t)n, cs));
+    if (launch_seam_compare((const SlicerHdr *const *)base, (const SlicerHdr *const *)(base + sizeof(void *) * room),
+                            (const int *)(base + 2 * sizeof(void *) * room), params_d.as<SlicerParams>(), mismatch_d.as<int>(), n, cs))
+        return -1;
+    stats.launches++;
+    NFC_CUDA_CHECK(cudaMemcpyAsync(mism.data(), mismatch_d.p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, cs));
+    return 0;
+}
+
+// NFC_SEGDEBUG: the cycles the streaming kernel spent on each segment (its final state's count, in thousands) and the
+// tiles it redid or took slowly (pad), on stderr.
+static int print_segment_cycles(const std::vector<SegWork> &works) {
+    const int nseg = (int)works.size();
+    double sum = 0;
+    uint32_t mn = ~0u, mx = 0;
+    std::vector<uint32_t> kc((size_t)nseg), rs((size_t)nseg);
+    for (int k = 0; k < nseg; k++) {
+        SlicerHdr h;
+        NFC_CUDA_CHECK(cudaMemcpy(&h, works[(size_t)k].state_out, sizeof(SlicerHdr), cudaMemcpyDeviceToHost));
+        kc[(size_t)k] = h.count; rs[(size_t)k] = h.pad;
+        sum += h.count; mn = std::min(mn, h.count); mx = std::max(mx, h.count);
+    }
+    fprintf(stderr, "segments %d kcycles min %u avg %.0f max %u\n", nseg, mn, sum / nseg, mx);
+    for (int k = 0; k < nseg; k += std::max(1, nseg / 24))
+        fprintf(stderr, "  seg %d: %u kcyc, redo %u slow %u\n", k, kc[(size_t)k], rs[(size_t)k] >> 16, rs[(size_t)k] & 0xffff);
+    // the slowest
+    for (int q = 0; q < 6; q++) {
+        int best = 0;
+        for (int k = 1; k < nseg; k++) if (kc[(size_t)k] > kc[(size_t)best]) best = k;
+        fprintf(stderr, "  slowest seg %d: %u kcyc, redo %u slow %u\n", best, kc[(size_t)best], rs[(size_t)best] >> 16, rs[(size_t)best] & 0xffff);
+        kc[(size_t)best] = 0;
+    }
+    return 0;
+}
+
+// Runs one slicer kernel over [a, b) of a slab and leaves the slab's true final state in `state`.  The streaming kernel
+// writes the class bitmap in place ([bm_lo, bm_hi) afterwards); the first-generation and the sequential kernel write
+// transition lists per segment, gathered into trans_dense[slab_seq & 1] (*R_out transitions).  *fell_back: a parallel
+// kernel left the exactly-summable regime, the caller redoes the slab with the sequential kernel.
+int Stream::run_slicer(Slicer kind, const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b,
                        uint32_t *R_out, bool *fell_back) {
+    // the slabs whose chains are still queued read the bitmap and trans_dense this slicer is about to overwrite; should one
+    // of them have to be done again, its input must still be there: look at them first (their chains end within a fraction
+    // of a millisecond)
+    if (finalize_all()) return -1;
+    bm_hi = bm_lo = 0;
+    const bool bitmap = kind == Slicer::streaming;
     const int L = sp.L;
     const int T = tile();
     *fell_back = false;
@@ -848,20 +915,26 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
     std::vector<int64_t> begins;  // first emitted sample of each segment
     begins.push_back(a);
     int64_t H = 0;
-    if (!serial) {
-        int64_t Hs = halo > 0 ? halo : (int64_t)16 * L;
+    if (kind != Slicer::sequential) {
+        const int64_t Hs = halo > 0 ? halo : (int64_t)16 * L;
         H = (Hs + T - 1) / T * T;
         int64_t S = seg_len;
         if (S <= 0) {
-            // as many segments as CTAs fit on the device at once (times k), each at least 6 halos long so that
-            // the speculative halo costs little, at most 256 windows so that a redo stays cheap
             const int64_t n = b - a, res = std::max(1, resident_ctas);
-            const int64_t s_min = 6 * H, s_max = std::max<int64_t>((int64_t)256 * L, s_min);
-            int64_t k = 1;
-            while (n / (res * (k + 1)) >= s_min) k++;
-            S = n / (res * k);
-            if (S < s_min) S = s_min;
-            if (S > s_max) S = s_max;
+            const int64_t s_min = 6 * H;
+            int64_t s_max, k = 1;
+            if (bitmap) {
+                // one segment per resident CTA if that keeps them below s_max, else the fewest waves that do: the longer
+                // the segments, the smaller the share of the speculative starts
+                s_max = std::max<int64_t>((int64_t)4096 * L, s_min);
+                k = std::max<int64_t>(1, (n + res * s_max - 1) / (res * s_max));
+            } else {
+                // as many segments as CTAs fit on the device at once (times k), each at least 6 halos long so that the
+                // speculative halo costs little, at most 256 windows so that a redo stays cheap
+                s_max = std::max<int64_t>((int64_t)256 * L, s_min);
+                while (n / (res * (k + 1)) >= s_min) k++;
+            }
+            S = std::clamp(n / (res * k), s_min, s_max);
         }
         S = (S + T - 1) / T * T;
         int64_t b1 = a + std::max<int64_t>(S, (int64_t)L + H);
@@ -876,14 +949,36 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
     const int NCK = 3;
     // checkpoints of every speculative segment, at 1, 3 and 7 halos after its first emitted sample
     const int64_t ck_off[NCK] = {H, 3 * H, 7 * H};
-    // state blocks: [seam_in k][state_out k] per segment
+    // state blocks: [seam_in k][state_out k] per segment; work items: the segments, behind them the redos of a repair round
     if (states_d.ensure(sblk * 2 * (size_t)nseg) || (nseg > 1 && ckpt_d.ensure(sblk * NCK * (size_t)nseg))) return -1;
-    if (seg_counts.ensure(sizeof(uint32_t) * (size_t)nseg) || seg_status.ensure(sizeof(int32_t) * (size_t)nseg) ||
-        works_d.ensure(sizeof(SegWork) * (size_t)nseg) || mismatch_d.ensure(sizeof(int) * (size_t)nseg) ||
-        seam_ptrs.ensure((sizeof(void *) * 2 + sizeof(int)) * (size_t)nseg))
+    if (seg_status.ensure(sizeof(int32_t) * (size_t)nseg) || works_d.ensure(sizeof(SegWork) * (size_t)nseg * 2) ||
+        mismatch_d.ensure(sizeof(int) * (size_t)nseg) || seam_ptrs.ensure((sizeof(void *) * 2 + sizeof(int)) * (size_t)nseg))
         return -1;
-    if (serial && serial_ring.ensure((size_t)L * 4 + 64)) return -1;
+    if (!bitmap && seg_counts.ensure(sizeof(uint32_t) * (size_t)nseg)) return -1;
+    if (kind == Slicer::sequential && serial_ring.ensure((size_t)L * 4 + 64)) return -1;
+    // bitmap of the slab, chunk 0 at the tile boundary at or before a
+    const int64_t bm_pos0 = a / T * T;
+    if (bitmap && bitmap_d.ensure(((size_t)((b - bm_pos0 + 127) / 128) + 64) * 32)) return -1;
+    auto seam_in = [&](int k) { return reinterpret_cast<SlicerHdr *>(states_d.as<char>() + sblk * (2 * (size_t)k)); };
+    auto st_out = [&](int k) { return reinterpret_cast<SlicerHdr *>(states_d.as<char>() + sblk * (2 * (size_t)k + 1)); };
+    auto ckpt = [&](int k, int j) { return reinterpret_cast<SlicerHdr *>(ckpt_d.as<char>() + sblk * ((size_t)k * NCK + (size_t)j)); };
+    auto tmp_state = [&](int i) { return reinterpret_cast<SlicerHdr *>(redo_states.as<char>() + sblk * (size_t)i); };
+    auto launch = [&](const SegWork *d_works, int n_works) -> int {
+        if (kind == Slicer::streaming) {
+            if (launch_streaming(d_works, n_works)) return -1;
+        } else if (kind == Slicer::first_gen) {
+            if (launch_slicer(d_works, n_works, params_d.as<SlicerParams>(), L, vec_ok(), cs)) return -1;
+        } else {
+            if (launch_slicer_serial(d_works, n_works, params_d.as<SlicerParams>(), serial_ring.as<float>(), (size_t)L + 16, cs))
+                return -1;
+            stats.serial_segments += n_works;
+        }
+        stats.launches++;
+        stats.slicer_launches++;
+        return 0;
+    };
 
+    // transition lists: capacities per segment, raised when a launch overflows them
     std::vector<uint32_t> caps((size_t)nseg);
     for (int k = 0; k < nseg; k++) {
         const int64_t e = k + 1 < nseg ? begins[(size_t)k + 1] : b;
@@ -898,18 +993,18 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
     };
 
     for (int attempt = 0; attempt < 4; attempt++) {
-        size_t total_cap = 0;
         std::vector<size_t> toff((size_t)nseg);
-        for (int k = 0; k < nseg; k++) {
-            toff[(size_t)k] = total_cap;
-            total_cap += caps[(size_t)k];
+        if (!bitmap) {
+            size_t total_cap = 0;
+            for (int k = 0; k < nseg; k++) {
+                toff[(size_t)k] = total_cap;
+                total_cap += caps[(size_t)k];
+            }
+            if (trans_seg.ensure(total_cap * sizeof(TransRec) + 16)) return -1;
         }
-        if (trans_seg.ensure(total_cap * sizeof(TransRec) + 16)) return -1;
-        auto seam_in = [&](int k) { return reinterpret_cast<SlicerHdr *>(states_d.as<char>() + sblk * (2 * (size_t)k)); };
-        auto st_out = [&](int k) { return reinterpret_cast<SlicerHdr *>(states_d.as<char>() + sblk * (2 * (size_t)k + 1)); };
-        auto ckpt = [&](int k, int j) { return reinterpret_cast<SlicerHdr *>(ckpt_d.as<char>() + sblk * ((size_t)k * NCK + (size_t)j)); };
         for (int k = 0; k < nseg; k++) {
             SegWork &w = works[(size_t)k];
+            memset(&w, 0, sizeof(w));
             w.in = d_in;
             w.in_pos0 = in_pos0;
             w.in_begin = in_begin;
@@ -926,57 +1021,35 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                 w.ckpt_state[j] = use ? ckpt(k, j) : nullptr;
             }
             w.state_out = st_out(k);
-            w.trans = trans_seg.as<TransRec>() + toff[(size_t)k];
-            w.trans_cap = caps[(size_t)k];
-            w.trans_count = seg_counts.as<uint32_t>() + k;
             w.status = seg_status.as<int32_t>() + k;
-            w.param_idx = 0;
-            w.pad = 0;
+            if (bitmap) {
+                w.bitmap = bitmap_d.as<uint32_t>();
+                w.bm_pos0 = bm_pos0;
+            } else {
+                w.trans = trans_seg.as<TransRec>() + toff[(size_t)k];
+                w.trans_cap = caps[(size_t)k];
+                w.trans_count = seg_counts.as<uint32_t>() + k;
+            }
         }
         NFC_CUDA_CHECK(cudaMemcpyAsync(works_d.p, works.data(), sizeof(SegWork) * (size_t)nseg, cudaMemcpyHostToDevice, cs));
-        if (serial) {
-            if (launch_slicer_serial(works_d.as<SegWork>(), nseg, params_d.as<SlicerParams>(), serial_ring.as<float>(),
-                                     (size_t)L + 16, cs))
-                return -1;
-            stats.serial_segments += nseg;
-        } else {
-            if (launch_slicer(works_d.as<SegWork>(), nseg, params_d.as<SlicerParams>(), L, vec_ok(), cs)) return -1;
-        }
-        stats.launches++;
-        stats.slicer_launches++;
+        if (launch(works_d.as<SegWork>(), nseg)) return -1;
         stats.segments += nseg;
 
         // ---- seams: compare what each speculative segment assumed with what its predecessor reached
         std::vector<int> mism((size_t)nseg, 0);
         std::vector<const SlicerHdr *> truth((size_t)nseg, nullptr), assumed((size_t)nseg, nullptr);
-        std::vector<int> pidx((size_t)nseg, 0);
-        char *sp_base = seam_ptrs.as<char>();
-        auto compare = [&](int n) -> int {
-            NFC_CUDA_CHECK(cudaMemcpyAsync(sp_base, truth.data(), sizeof(void *) * (size_t)n, cudaMemcpyHostToDevice, cs));
-            NFC_CUDA_CHECK(cudaMemcpyAsync(sp_base + sizeof(void *) * (size_t)nseg, assumed.data(), sizeof(void *) * (size_t)n,
-                                           cudaMemcpyHostToDevice, cs));
-            NFC_CUDA_CHECK(cudaMemcpyAsync(sp_base + 2 * sizeof(void *) * (size_t)nseg, pidx.data(), sizeof(int) * (size_t)n,
-                                           cudaMemcpyHostToDevice, cs));
-            NFC_CUDA_CHECK(cudaMemsetAsync(mismatch_d.p, 0, sizeof(int) * (size_t)n, cs));
-            if (launch_seam_compare((const SlicerHdr *const *)sp_base,
-                                    (const SlicerHdr *const *)(sp_base + sizeof(void *) * (size_t)nseg),
-                                    (const int *)(sp_base + 2 * sizeof(void *) * (size_t)nseg), params_d.as<SlicerParams>(),
-                                    mismatch_d.as<int>(), n, cs))
-                return -1;
-            stats.launches++;
-            NFC_CUDA_CHECK(cudaMemcpyAsync(mism.data(), mismatch_d.p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, cs));
-            return 0;
-        };
         if (nseg > 1) {
             for (int k = 1; k < nseg; k++) {
                 truth[(size_t)k] = st_out(k - 1);
                 assumed[(size_t)k] = seam_in(k);
             }
-            if (compare(nseg)) return -1;
+            if (compare_states(truth, assumed, nseg, mism)) return -1;
         }
-        NFC_CUDA_CHECK(cudaMemcpyAsync(counts.data(), seg_counts.p, sizeof(uint32_t) * (size_t)nseg, cudaMemcpyDeviceToHost, cs));
+        if (!bitmap)
+            NFC_CUDA_CHECK(cudaMemcpyAsync(counts.data(), seg_counts.p, sizeof(uint32_t) * (size_t)nseg, cudaMemcpyDeviceToHost, cs));
         NFC_CUDA_CHECK(cudaMemcpyAsync(status.data(), seg_status.p, sizeof(int32_t) * (size_t)nseg, cudaMemcpyDeviceToHost, cs));
         NFC_CUDA_CHECK(sync_cs());
+        if (bitmap) add_kernel_time();
         int st_all = 0;
         bool over = false;
         for (int k = 0; k < nseg; k++) {
@@ -986,8 +1059,8 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                 caps[(size_t)k] = counts[(size_t)k] + 16;
             }
         }
-        if (!serial && (st_all & (SEG_INEXACT | SEG_NOT_SANE))) {
-            *fell_back = true;  // caller redoes the slab with the sequential kernel
+        if (kind != Slicer::sequential && (st_all & (SEG_INEXACT | SEG_NOT_SANE))) {
+            *fell_back = true;
             return 0;
         }
         if (over) {
@@ -997,10 +1070,12 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
 
         // ---- repair: a segment whose assumption was wrong is redone from its predecessor's true final state,
         // checkpoint by checkpoint, and stops as soon as it reproduces a checkpoint of the speculative run: from
-        // there on the speculative output is the true output.  Only a redo that reaches the segment end changes
-        // the segment's final state, and then the next seam is checked again.
+        // there on the speculative output is the true output.  Only a redo that reaches the segment end changes the
+        // segment's final state, and then the next seam is checked again.  A redo of the streaming kernel overwrites the
+        // bitmap in place; the other kernels' redos write to redo_trans, and `pieces` says which stretches of which lists
+        // make up each segment's transitions.
         std::vector<std::vector<Piece>> pieces((size_t)nseg);
-        for (int k = 0; k < nseg; k++) pieces[(size_t)k].push_back(Piece{works[(size_t)k].trans, counts[(size_t)k]});
+        for (int k = 0; k < nseg && !bitmap; k++) pieces[(size_t)k].push_back(Piece{works[(size_t)k].trans, counts[(size_t)k]});
         std::vector<char> bad((size_t)nseg, 0);
         int nbad = 0;
         for (int k = 1; k < nseg; k++) {
@@ -1020,11 +1095,10 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                 roff[(size_t)i] = rcap_total;
                 rcap_total += caps[(size_t)ks[(size_t)i]];
             }
-            if (redo_states.ensure(sblk * (size_t)nr) || redo_trans.ensure(rcap_total * sizeof(TransRec) + 16) ||
-                redo_counts.ensure(sizeof(uint32_t) * 2 * (size_t)nr) || works_d.ensure(sizeof(SegWork) * ((size_t)nseg + (size_t)nr)))
+            // redo_counts: the redos' transition counts, then their status
+            if (redo_states.ensure(sblk * (size_t)nr) || redo_counts.ensure(sizeof(uint32_t) * 2 * (size_t)nr) ||
+                (!bitmap && redo_trans.ensure(rcap_total * sizeof(TransRec) + 16)))
                 return -1;
-            NFC_CUDA_CHECK(cudaMemcpyAsync(works_d.p, works.data(), sizeof(SegWork) * (size_t)nseg, cudaMemcpyHostToDevice, cs));
-            auto tmp_state = [&](int i) { return reinterpret_cast<SlicerHdr *>(redo_states.as<char>() + sblk * (size_t)i); };
             std::vector<uint32_t> used((size_t)nr, 0);
             std::vector<int64_t> at((size_t)nr);
             std::vector<char> active((size_t)nr, 1);
@@ -1036,28 +1110,27 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                     if (!active[(size_t)i]) continue;
                     const int k = ks[(size_t)i];
                     const SegWork &ws = works[(size_t)k];
-                    const int64_t target = (stage < NCK && ws.ckpt_state[stage]) ? ws.ckpt_pos[stage] : ws.end;
                     if (stage < NCK && !ws.ckpt_state[stage]) continue;  // no such checkpoint: a later stage runs on
                     SegWork w = ws;
                     w.warm_begin = w.begin = at[(size_t)i];
-                    w.end = target;
+                    w.end = stage < NCK ? ws.ckpt_pos[stage] : ws.end;
                     w.state_in = at[(size_t)i] == ws.begin ? st_out(k - 1) : tmp_state(i);
                     w.seam_in = nullptr;
                     for (int j = 0; j < NCK; j++) { w.ckpt_pos[j] = INT64_MAX; w.ckpt_state[j] = nullptr; }
                     w.state_out = tmp_state(i);
-                    w.trans = redo_trans.as<TransRec>() + roff[(size_t)i] + used[(size_t)i];
-                    w.trans_cap = caps[(size_t)k] - std::min(caps[(size_t)k], used[(size_t)i]);
-                    w.trans_count = redo_counts.as<uint32_t>() + i;
                     w.status = reinterpret_cast<int32_t *>(redo_counts.as<uint32_t>() + nr + i);
+                    if (!bitmap) {
+                        w.trans = redo_trans.as<TransRec>() + roff[(size_t)i] + used[(size_t)i];
+                        w.trans_cap = caps[(size_t)k] - std::min(caps[(size_t)k], used[(size_t)i]);
+                        w.trans_count = redo_counts.as<uint32_t>() + i;
+                    }
                     redo.push_back(w);
                     who.push_back(i);
                 }
                 if (redo.empty()) continue;
                 SegWork *d_redo = works_d.as<SegWork>() + nseg;
                 NFC_CUDA_CHECK(cudaMemcpyAsync(d_redo, redo.data(), sizeof(SegWork) * redo.size(), cudaMemcpyHostToDevice, cs));
-                if (launch_slicer(d_redo, (int)redo.size(), params_d.as<SlicerParams>(), L, vec_ok(), cs)) return -1;
-                stats.launches++;
-                stats.slicer_launches++;
+                if (launch(d_redo, (int)redo.size())) return -1;
                 // did each redo reproduce the checkpoint it stopped at?
                 const int nw = (int)who.size();
                 std::vector<SlicerHdr> ck_hdr((size_t)nw);
@@ -1065,37 +1138,41 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                     const int i = who[(size_t)q], k = ks[(size_t)i];
                     truth[(size_t)q] = tmp_state(i);
                     assumed[(size_t)q] = stage < NCK ? works[(size_t)k].ckpt_state[stage] : tmp_state(i);
-                    pidx[(size_t)q] = 0;
-                    if (stage < NCK)
+                    if (!bitmap && stage < NCK)
                         NFC_CUDA_CHECK(cudaMemcpyAsync(&ck_hdr[(size_t)q], works[(size_t)k].ckpt_state[stage], sizeof(SlicerHdr),
                                                        cudaMemcpyDeviceToHost, cs));
                 }
-                if (compare(nw)) return -1;
+                if (compare_states(truth, assumed, nw, mism)) return -1;
                 std::vector<uint32_t> rc((size_t)nr * 2);
                 NFC_CUDA_CHECK(cudaMemcpyAsync(rc.data(), redo_counts.p, sizeof(uint32_t) * 2 * (size_t)nr, cudaMemcpyDeviceToHost, cs));
                 NFC_CUDA_CHECK(sync_cs());
+                if (bitmap) add_kernel_time();
                 for (int q = 0; q < nw; q++) {
                     const int i = who[(size_t)q], k = ks[(size_t)i];
-                    const uint32_t got = rc[(size_t)i];
-                    if (got > redo[(size_t)q].trans_cap) {
-                        over = true;
-                        caps[(size_t)k] = caps[(size_t)k] * 2 + got;
+                    if ((int32_t)rc[(size_t)nr + i] & (SEG_INEXACT | SEG_NOT_SANE)) {
+                        *fell_back = true;
+                        return 0;
                     }
-                    used[(size_t)i] += std::min(got, redo[(size_t)q].trans_cap);
+                    if (!bitmap) {
+                        const uint32_t got = rc[(size_t)i];
+                        if (got > redo[(size_t)q].trans_cap) {
+                            over = true;
+                            caps[(size_t)k] = caps[(size_t)k] * 2 + got;
+                        }
+                        used[(size_t)i] += std::min(got, redo[(size_t)q].trans_cap);
+                    }
                     at[(size_t)i] = redo[(size_t)q].end;
-                    const TransRec *rbase = redo_trans.as<TransRec>() + roff[(size_t)i];
                     if (stage < NCK && !mism[(size_t)q]) {
                         // converged with the speculative run: keep its output from this checkpoint on
                         const uint32_t cc = ck_hdr[(size_t)q].count;
-                        pieces[(size_t)k].clear();
-                        pieces[(size_t)k].push_back(Piece{rbase, used[(size_t)i]});
-                        pieces[(size_t)k].push_back(Piece{works[(size_t)k].trans + cc, counts[(size_t)k] - std::min(counts[(size_t)k], cc)});
+                        if (!bitmap)
+                            pieces[(size_t)k] = {Piece{redo_trans.as<TransRec>() + roff[(size_t)i], used[(size_t)i]},
+                                                 Piece{works[(size_t)k].trans + cc, counts[(size_t)k] - std::min(counts[(size_t)k], cc)}};
                         active[(size_t)i] = 0;
                         bad[(size_t)k] = 0;
                     } else if (stage == NCK || at[(size_t)i] >= works[(size_t)k].end) {
                         // redone to its end: new final state, next seam must be looked at again
-                        pieces[(size_t)k].clear();
-                        pieces[(size_t)k].push_back(Piece{rbase, used[(size_t)i]});
+                        if (!bitmap) pieces[(size_t)k] = {Piece{redo_trans.as<TransRec>() + roff[(size_t)i], used[(size_t)i]}};
                         NFC_CUDA_CHECK(cudaMemcpyAsync(st_out(k), tmp_state(i), sblk, cudaMemcpyDeviceToDevice, cs));
                         active[(size_t)i] = 0;
                         bad[(size_t)k] = 0;
@@ -1113,15 +1190,14 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                 for (size_t q = 0; q < unk.size(); q++) {
                     truth[q] = st_out(unk[q] - 1);
                     assumed[q] = seam_in(unk[q]);
-                    pidx[q] = 0;
                 }
-                if (compare((int)unk.size())) return -1;
+                if (compare_states(truth, assumed, (int)unk.size(), mism)) return -1;
                 NFC_CUDA_CHECK(sync_cs());
                 for (size_t q = 0; q < unk.size(); q++) bad[(size_t)unk[q]] = mism[q] ? 1 : 0;
             }
             nbad = 0;
             for (int k = 1; k < nseg; k++) nbad += bad[(size_t)k] ? 1 : 0;
-            if (nbad > 0) {
+            if (nbad > 0 && !bitmap) {
                 // another round will overwrite redo_trans / redo_states: detach the buffers this round's pieces use
                 kept_bufs.push_back(redo_trans);
                 redo_trans = DevBuf();
@@ -1136,6 +1212,15 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
         if (nbad > 0) {
             set_error("seam repair did not settle");
             return -1;
+        }
+        if (bitmap && getenv("NFC_SEGDEBUG") && print_segment_cycles(works)) return -1;
+        // the slab's final state becomes the stream's state
+        NFC_CUDA_CHECK(cudaMemcpyAsync(state.p, st_out(nseg - 1), sblk, cudaMemcpyDeviceToDevice, cs));
+        if (bitmap) {
+            bm_lo = a;
+            bm_hi = b;
+            bm_origin = bm_pos0;
+            return 0;
         }
         // ---- dense ordered transitions
         std::vector<const TransRec *> psrc;
@@ -1159,8 +1244,6 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
                                  (const uint32_t *)(pb + np * (sizeof(void *) + 4)), (int)np, td.as<TransRec>(), cs))
             return -1;
         stats.launches++;
-        // the slab's final state becomes the stream's state
-        NFC_CUDA_CHECK(cudaMemcpyAsync(state.p, st_out(nseg - 1), sblk, cudaMemcpyDeviceToDevice, cs));
         NFC_CUDA_CHECK(sync_cs());  // pieces may live in buffers released below
         for (DevBuf &kb : kept_bufs) kb.release();
         kept_bufs.clear();
@@ -1169,265 +1252,6 @@ int Stream::run_slicer(const void *d_in, int64_t in_pos0, int64_t in_begin, int6
     }
     set_error("transition buffers kept overflowing");
     return -1;
-}
-
-// The streaming kernel over [a, b): class bitmap (fixed-rate output, no per-segment lists), seams verified and repaired like
-// run_slicer, then the dense ordered transitions of [a, b_post) extracted from the bitmap (b_post <= b: the slicer may cover
-// several slabs at once -- longer segments, relatively shorter speculative starts; extract_only serves the rest).
-int Stream::run_slicer_bm(const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b, bool *fell_back) {
-    // the slabs whose chains are still queued read the bitmap this launch is about to overwrite; should one of them have to be
-    // done again, its bitmap must still be there: look at them first (their chains end within a fraction of a millisecond)
-    if (finalize_all()) return -1;
-    bm_hi = bm_lo = 0;
-    const int L = sp.L;
-    const int T = tile();
-    *fell_back = false;
-    // ---- plan segments (as run_slicer)
-    std::vector<int64_t> begins;
-    begins.push_back(a);
-    const int64_t Hs = halo > 0 ? halo : (int64_t)16 * L;
-    const int64_t H = (Hs + T - 1) / T * T;
-    {
-        int64_t S = seg_len;
-        if (S <= 0) {
-            const int64_t n = b - a, res = std::max(1, resident_ctas);
-            // one segment per resident CTA if that keeps them below s_max, else the fewest waves that do: the longer the
-            // segments, the smaller the share of the speculative starts
-            const int64_t s_min = 6 * H, s_max = std::max<int64_t>((int64_t)4096 * L, s_min);
-            const int64_t k = std::max<int64_t>(1, (n + res * s_max - 1) / (res * s_max));
-            S = n / (res * k);
-            if (S < s_min) S = s_min;
-            if (S > s_max) S = s_max;
-        }
-        S = (S + T - 1) / T * T;
-        int64_t b1 = a + std::max<int64_t>(S, (int64_t)L + H);
-        b1 = (b1 + T - 1) / T * T;
-        while (b1 + S / 2 <= b && b1 < b) {
-            begins.push_back(b1);
-            b1 += S;
-        }
-    }
-    const int nseg = (int)begins.size();
-    const size_t sblk = state_block_bytes(L);
-    const int NCK = 3;
-    const int64_t ck_off[NCK] = {H, 3 * H, 7 * H};
-    if (states_d.ensure(sblk * 2 * (size_t)nseg) || (nseg > 1 && ckpt_d.ensure(sblk * NCK * (size_t)nseg))) return -1;
-    if (seg_status.ensure(sizeof(int32_t) * (size_t)nseg) || works_d.ensure(sizeof(SegWork) * (size_t)nseg * 2) ||
-        mismatch_d.ensure(sizeof(int) * (size_t)nseg) || seam_ptrs.ensure((sizeof(void *) * 2 + sizeof(int)) * (size_t)nseg))
-        return -1;
-    // bitmap of the slab, chunk 0 at the tile boundary at or before a
-    const int64_t bm_pos0 = a / T * T;
-    const size_t n_chunks = (size_t)((b - bm_pos0 + 127) / 128);
-    if (bitmap_d.ensure((n_chunks + 64) * 32)) return -1;
-
-    std::vector<SegWork> works((size_t)nseg);
-    std::vector<int32_t> status((size_t)nseg);
-    auto seam_in = [&](int k) { return reinterpret_cast<SlicerHdr *>(states_d.as<char>() + sblk * (2 * (size_t)k)); };
-    auto st_out = [&](int k) { return reinterpret_cast<SlicerHdr *>(states_d.as<char>() + sblk * (2 * (size_t)k + 1)); };
-    auto ckpt = [&](int k, int j) { return reinterpret_cast<SlicerHdr *>(ckpt_d.as<char>() + sblk * ((size_t)k * NCK + (size_t)j)); };
-    for (int k = 0; k < nseg; k++) {
-        SegWork &w = works[(size_t)k];
-        memset(&w, 0, sizeof(w));
-        w.in = d_in;
-        w.in_pos0 = in_pos0;
-        w.in_begin = in_begin;
-        w.in_end = in_end;
-        w.begin = begins[(size_t)k];
-        w.end = k + 1 < nseg ? begins[(size_t)k + 1] : b;
-        w.warm_begin = k == 0 ? a : w.begin - H;
-        w.slab_pos0 = a;
-        w.state_in = k == 0 ? state.as<SlicerHdr>() : nullptr;
-        w.seam_in = k == 0 ? nullptr : seam_in(k);
-        for (int j = 0; j < NCK; j++) {
-            const bool use = k > 0 && w.begin + ck_off[j] < w.end;
-            w.ckpt_pos[j] = use ? w.begin + ck_off[j] : INT64_MAX;
-            w.ckpt_state[j] = use ? ckpt(k, j) : nullptr;
-        }
-        w.state_out = st_out(k);
-        w.trans = nullptr;
-        w.trans_cap = 0;
-        w.trans_count = nullptr;
-        w.status = seg_status.as<int32_t>() + k;
-        w.param_idx = 0;
-        w.bitmap = bitmap_d.as<uint32_t>();
-        w.bm_pos0 = bm_pos0;
-    }
-    NFC_CUDA_CHECK(cudaMemcpyAsync(works_d.p, works.data(), sizeof(SegWork) * (size_t)nseg, cudaMemcpyHostToDevice, cs));
-    NFC_CUDA_CHECK(cudaEventRecord(ev_k0, cs));
-    if (launch_slicer_streaming(works_d.as<SegWork>(), nseg, params_d.as<SlicerParams>(), L, sp.input_kind, cs)) return -1;
-    NFC_CUDA_CHECK(cudaEventRecord(ev_k1, cs));
-    stats.launches++;
-    stats.slicer_launches++;
-    stats.segments += nseg;
-    auto kernel_time = [&]() {  // after a synchronisation of the stream
-        float ms = 0;
-        if (cudaEventElapsedTime(&ms, ev_k0, ev_k1) == cudaSuccess) {
-            stats.slicer_kernel_ms += ms;
-            stats.slicer_kernel_launches++;
-        }
-    };
-
-    // ---- seams
-    std::vector<int> mism((size_t)nseg, 0);
-    std::vector<const SlicerHdr *> truth((size_t)nseg, nullptr), assumed((size_t)nseg, nullptr);
-    std::vector<int> pidx((size_t)nseg, 0);
-    char *sp_base = seam_ptrs.as<char>();
-    auto compare = [&](int n) -> int {
-        NFC_CUDA_CHECK(cudaMemcpyAsync(sp_base, truth.data(), sizeof(void *) * (size_t)n, cudaMemcpyHostToDevice, cs));
-        NFC_CUDA_CHECK(cudaMemcpyAsync(sp_base + sizeof(void *) * (size_t)nseg, assumed.data(), sizeof(void *) * (size_t)n,
-                                       cudaMemcpyHostToDevice, cs));
-        NFC_CUDA_CHECK(cudaMemcpyAsync(sp_base + 2 * sizeof(void *) * (size_t)nseg, pidx.data(), sizeof(int) * (size_t)n,
-                                       cudaMemcpyHostToDevice, cs));
-        NFC_CUDA_CHECK(cudaMemsetAsync(mismatch_d.p, 0, sizeof(int) * (size_t)n, cs));
-        if (launch_seam_compare((const SlicerHdr *const *)sp_base, (const SlicerHdr *const *)(sp_base + sizeof(void *) * (size_t)nseg),
-                                (const int *)(sp_base + 2 * sizeof(void *) * (size_t)nseg), params_d.as<SlicerParams>(),
-                                mismatch_d.as<int>(), n, cs))
-            return -1;
-        stats.launches++;
-        NFC_CUDA_CHECK(cudaMemcpyAsync(mism.data(), mismatch_d.p, sizeof(int) * (size_t)n, cudaMemcpyDeviceToHost, cs));
-        return 0;
-    };
-    if (nseg > 1) {
-        for (int k = 1; k < nseg; k++) {
-            truth[(size_t)k] = st_out(k - 1);
-            assumed[(size_t)k] = seam_in(k);
-        }
-        if (compare(nseg)) return -1;
-    }
-    NFC_CUDA_CHECK(cudaMemcpyAsync(status.data(), seg_status.p, sizeof(int32_t) * (size_t)nseg, cudaMemcpyDeviceToHost, cs));
-    NFC_CUDA_CHECK(sync_cs());
-    kernel_time();
-    int st_all = 0;
-    for (int k = 0; k < nseg; k++) st_all |= status[(size_t)k];
-    if (st_all & (SEG_INEXACT | SEG_NOT_SANE)) {
-        *fell_back = true;  // caller redoes the slab with the sequential kernel
-        return 0;
-    }
-    // ---- repair: redo a wrong segment from its predecessor's true final state, checkpoint by checkpoint; the
-    // redo overwrites the bitmap in place and stops at the first checkpoint of the speculative run it reproduces
-    std::vector<char> bad((size_t)nseg, 0);
-    int nbad = 0;
-    for (int k = 1; k < nseg; k++) {
-        bad[(size_t)k] = mism[(size_t)k] ? 1 : 0;
-        nbad += bad[(size_t)k];
-    }
-    for (int guard = 0; nbad > 0 && guard < nseg + 2; guard++) {
-        std::vector<int> ks;
-        for (int k = 1; k < nseg; k++)
-            if (bad[(size_t)k] && !bad[(size_t)k - 1]) ks.push_back(k);
-        const int nr = (int)ks.size();
-        stats.seam_mismatches += nr;
-        if (redo_states.ensure(sblk * (size_t)nr) || redo_counts.ensure(sizeof(int32_t) * (size_t)nr)) return -1;
-        auto tmp_state = [&](int i) { return reinterpret_cast<SlicerHdr *>(redo_states.as<char>() + sblk * (size_t)i); };
-        std::vector<int64_t> at((size_t)nr);
-        std::vector<char> active((size_t)nr, 1);
-        for (int i = 0; i < nr; i++) at[(size_t)i] = works[(size_t)ks[(size_t)i]].begin;
-        for (int stage = 0; stage <= NCK; stage++) {
-            std::vector<SegWork> redo;
-            std::vector<int> who;
-            for (int i = 0; i < nr; i++) {
-                if (!active[(size_t)i]) continue;
-                const int k = ks[(size_t)i];
-                const SegWork &ws = works[(size_t)k];
-                if (stage < NCK && !ws.ckpt_state[stage]) continue;  // no such checkpoint: a later stage runs on
-                const int64_t target = stage < NCK ? ws.ckpt_pos[stage] : ws.end;
-                SegWork w = ws;
-                w.warm_begin = w.begin = at[(size_t)i];
-                w.end = target;
-                w.state_in = at[(size_t)i] == ws.begin ? st_out(k - 1) : tmp_state(i);
-                w.seam_in = nullptr;
-                for (int j = 0; j < NCK; j++) { w.ckpt_pos[j] = INT64_MAX; w.ckpt_state[j] = nullptr; }
-                w.state_out = tmp_state(i);
-                w.status = redo_counts.as<int32_t>() + i;
-                redo.push_back(w);
-                who.push_back(i);
-            }
-            if (redo.empty()) continue;
-            SegWork *d_redo = works_d.as<SegWork>() + nseg;
-            NFC_CUDA_CHECK(cudaMemcpyAsync(d_redo, redo.data(), sizeof(SegWork) * redo.size(), cudaMemcpyHostToDevice, cs));
-            NFC_CUDA_CHECK(cudaEventRecord(ev_k0, cs));
-            if (launch_slicer_streaming(d_redo, (int)redo.size(), params_d.as<SlicerParams>(), L, sp.input_kind, cs)) return -1;
-            NFC_CUDA_CHECK(cudaEventRecord(ev_k1, cs));
-            stats.launches++;
-            stats.slicer_launches++;
-            const int nw = (int)who.size();
-            for (int q = 0; q < nw; q++) {
-                const int i = who[(size_t)q], k = ks[(size_t)i];
-                truth[(size_t)q] = tmp_state(i);
-                assumed[(size_t)q] = stage < NCK ? works[(size_t)k].ckpt_state[stage] : tmp_state(i);
-                pidx[(size_t)q] = 0;
-            }
-            if (compare(nw)) return -1;
-            std::vector<int32_t> rst((size_t)nr, 0);
-            NFC_CUDA_CHECK(cudaMemcpyAsync(rst.data(), redo_counts.p, sizeof(int32_t) * (size_t)nr, cudaMemcpyDeviceToHost, cs));
-            NFC_CUDA_CHECK(sync_cs());
-            kernel_time();
-            for (int q = 0; q < nw; q++) {
-                const int i = who[(size_t)q], k = ks[(size_t)i];
-                if (rst[(size_t)i] & (SEG_INEXACT | SEG_NOT_SANE)) {
-                    *fell_back = true;
-                    return 0;
-                }
-                at[(size_t)i] = redo[(size_t)q].end;
-                if (stage < NCK && !mism[(size_t)q]) {
-                    active[(size_t)i] = 0;  // converged with the speculative run: its bitmap from here on is the true one
-                    bad[(size_t)k] = 0;
-                } else if (stage == NCK || at[(size_t)i] >= works[(size_t)k].end) {
-                    NFC_CUDA_CHECK(cudaMemcpyAsync(st_out(k), tmp_state(i), sblk, cudaMemcpyDeviceToDevice, cs));
-                    active[(size_t)i] = 0;
-                    bad[(size_t)k] = 0;
-                    if (k + 1 < nseg) bad[(size_t)k + 1] = 2;  // unknown: re-compare below
-                }
-            }
-        }
-        std::vector<int> unk;
-        for (int k = 1; k < nseg; k++)
-            if (bad[(size_t)k] == 2) unk.push_back(k);
-        if (!unk.empty()) {
-            for (size_t q = 0; q < unk.size(); q++) {
-                truth[q] = st_out(unk[q] - 1);
-                assumed[q] = seam_in(unk[q]);
-                pidx[q] = 0;
-            }
-            if (compare((int)unk.size())) return -1;
-            NFC_CUDA_CHECK(sync_cs());
-            for (size_t q = 0; q < unk.size(); q++) bad[(size_t)unk[q]] = mism[q] ? 1 : 0;
-        }
-        nbad = 0;
-        for (int k = 1; k < nseg; k++) nbad += bad[(size_t)k] ? 1 : 0;
-    }
-    if (nbad > 0) {
-        set_error("seam repair did not settle");
-        return -1;
-    }
-
-    if (getenv("NFC_SEGDEBUG")) {
-        std::vector<char> blk(sblk);
-        double sum = 0;
-        uint32_t mn = ~0u, mx = 0;
-        std::vector<uint32_t> kc((size_t)nseg), rs((size_t)nseg);
-        for (int k = 0; k < nseg; k++) {
-            NFC_CUDA_CHECK(cudaMemcpy(blk.data(), st_out(k), sizeof(SlicerHdr), cudaMemcpyDeviceToHost));
-            const SlicerHdr *h = reinterpret_cast<const SlicerHdr *>(blk.data());
-            kc[(size_t)k] = h->count; rs[(size_t)k] = h->pad;
-            sum += h->count; mn = std::min(mn, h->count); mx = std::max(mx, h->count);
-        }
-        fprintf(stderr, "segments %d kcycles min %u avg %.0f max %u\n", nseg, mn, sum / nseg, mx);
-        for (int k = 0; k < nseg; k += std::max(1, nseg / 24))
-            fprintf(stderr, "  seg %d: %u kcyc, redo %u slow %u\n", k, kc[(size_t)k], rs[(size_t)k] >> 16, rs[(size_t)k] & 0xffff);
-        // the slowest
-        for (int q = 0; q < 6; q++) {
-            int best = 0;
-            for (int k = 1; k < nseg; k++) if (kc[(size_t)k] > kc[(size_t)best]) best = k;
-            fprintf(stderr, "  slowest seg %d: %u kcyc, redo %u slow %u\n", best, kc[(size_t)best], rs[(size_t)best] >> 16, rs[(size_t)best] & 0xffff);
-            kc[(size_t)best] = 0;
-        }
-    }
-    NFC_CUDA_CHECK(cudaMemcpyAsync(state.p, st_out(nseg - 1), sblk, cudaMemcpyDeviceToDevice, cs));
-    bm_lo = a;
-    bm_hi = b;
-    bm_origin = bm_pos0;
-    return 0;
 }
 
 static double now_ms() {
@@ -1491,21 +1315,18 @@ int Stream::process_slab(const void *d_in, int64_t in_pos0, int64_t in_begin, in
     NFC_CUDA_CHECK(cudaEventRecord(ev_a[ci], cs));
     uint32_t R = 0;
     bool fell_back = false, from_bitmap = false;
-    const bool par = parallel_ok();
     if (streaming_ok() && a >= bm_lo && b <= bm_hi) {
         from_bitmap = true;  // the slicer ran over this slab together with the one before
     } else if (streaming_ok()) {
-        if (run_slicer_bm(d_in, in_pos0, in_begin, in_end, a, std::max(b, slicer_end), &fell_back)) return -1;
+        if (run_slicer(Slicer::streaming, d_in, in_pos0, in_begin, in_end, a, std::max(b, slicer_end), &R, &fell_back)) return -1;
         from_bitmap = !fell_back;
     } else {
-        if (finalize_all()) return -1;  // trans_dense is written by this slab's slicer while an older chain may still read it
-        if (run_slicer(d_in, in_pos0, in_begin, in_end, a, b, !par, &R, &fell_back)) return -1;
+        const Slicer kind = parallel_ok() ? Slicer::first_gen : Slicer::sequential;
+        if (run_slicer(kind, d_in, in_pos0, in_begin, in_end, a, b, &R, &fell_back)) return -1;
     }
     if (fell_back) {
-        if (finalize_all()) return -1;
-        bm_lo = bm_hi = 0;
         serial_mode = true;  // sums are no longer exactly representable: stay on the sequential kernel
-        if (run_slicer(d_in, in_pos0, in_begin, in_end, a, b, true, &R, &fell_back)) return -1;
+        if (run_slicer(Slicer::sequential, d_in, in_pos0, in_begin, in_end, a, b, &R, &fell_back)) return -1;
     }
     return post_chain(a, b, from_bitmap, R, false, t0, now_ms());
 }

@@ -107,8 +107,8 @@ int64_t nfc_stream_push(nfc_stream *s, const void *items, int64_t n, int mem, in
  * in one space: capture = pos / *pitch, item index inside the capture = pos % *pitch (*pitch: items_per_capture rounded
  * up to whole tiles).  Events and symbols at indices below av_window or from items_per_capture on belong to no capture
  * (they flush the decoders between captures) and are to be skipped by the consumer; frames never carry such positions.
- * NFC_OUT_DROPPED_EVENTS is not available in this mode.  Needs av_window >= 1024 (a multiple of 4) and 16-byte aligned
- * captures.  Returns n_captures; -1 on error; -3 when some capture has to take the sequential path (negative or widely
+ * NFC_OUT_DROPPED_EVENTS is not available in this mode.  Needs av_window in [1024, 52000], a multiple of 4, and 16-byte
+ * aligned captures.  Returns n_captures; -1 on error; -3 when some capture has to take the sequential path (negative or widely
  * spread samples): decode the captures one by one with nfc_stream_push then.  The stream takes no further items until reset. */
 int64_t nfc_stream_push_batch(nfc_stream *s, const void *items, int mem, int64_t n_captures, int64_t items_per_capture,
                               int64_t stride_items, const double *lo_vals, const double *hi_vals, int64_t *pitch);

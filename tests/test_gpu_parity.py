@@ -373,6 +373,27 @@ def test_streaming_kernel_corner_cases(L, mx, tuning):
     print("stats", st)
 
 
+@pytest.mark.parametrize("L,streaming", [(52000, True), (51456, True), (51998, False)])
+def test_longest_parallel_windows(L, streaming):
+    """The top of the parallel window range, several segments each: a multiple of 4 up to 52000 takes the streaming kernel
+    (at 52000 the ring, the staging tile and the kernel's static scratch fill one CTA's shared memory), any other window
+    the first-generation kernel."""
+    mx = 339
+    # pauses at 1e-3 rather than 1e-4: the first-generation kernel starts a segment from the raw previous L samples, and at
+    # these windows its sums are exact only while those span at most 28 - 16 - 1 = 11 binades (else the sequential kernel)
+    x = np.maximum(_corner_stream(L, mx, 1_500_000, L + mx), np.float32(1e-3))
+    want = oracle.decode_capture(x, 13.56e6, hi_val=1.09, av_window=L, max_len=mx)
+    got = gpu_decode(x, 13.56e6, hi_val=1.09, av_window=L, max_len=mx, tuning=dict(seg_len=262144, halo=4 * L))
+    check_against_oracle(got, want)
+    st = got["stream"].stats()
+    assert not got["stream"].state()[0].serial_mode
+    assert st["segments"] >= 3
+    if streaming:
+        assert st["slicer_kernel_launches"] > 0
+    else:
+        assert st["slicer_kernel_launches"] == 0 and st["serial_segments"] == 0
+
+
 def test_streaming_kernel_degenerate_inputs():
     L, mx = 8192, 50
     # silence (ss == 0), then a carrier, negative samples, back to silence

@@ -34,7 +34,7 @@ namespace nfc {
 
 static const unsigned FULL = 0xffffffffu;
 // tile counters (device-wide): 0 streamed, 1 exact path, 2 coarse-step retries exhausted, 3 exact fix-point pass, 4 ring resums,
-// 5 repeated passes, 6 hysteresis risk, 7 fix-point pass gave up, 8 exact-path rounds, 9/10 first-generation kernel: refined / refine failed
+// 5 repeated passes, 6 hysteresis risk, 7 fix-point pass gave up, 8 exact-path rounds, 11-15 pipelined mode and cycles (slicer_fast.cuh)
 __device__ unsigned long long g_tile_stats[16];
 #ifdef NFC_CYCLES
 __device__ unsigned long long g_cyc[12];  // diagnostics build: see slicer_fast.cuh
@@ -85,8 +85,6 @@ __device__ __forceinline__ float load_one(const void *in, int64_t idx, const Sli
         }
     }
 }
-
-__device__ __forceinline__ int item_size(int kind) { return kind == IN_IQ_F32 ? 8 : (kind == IN_PCM_S16 ? 2 : 4); }
 
 // streaming 128-bit load: the sample stream is read exactly once
 __device__ __forceinline__ float4 ldg_stream4(const float4 *ptr) {
@@ -171,22 +169,7 @@ __device__ __forceinline__ bool st2_forced(int64_t i, int64_t b, int64_t a, int 
 }
 
 // ---------------------------------------------------------------- block-wide primitives
-struct RowRec {      // one warp x one row of a tile (128 samples), positions relative to the tile start
-    int first;       // (first_pos << 2) | (val + 1) of the first active sample, INT_MAX when the row part is empty
-    int last;        // (last_pos << 2) | (val + 1) of the last active sample, -1 when empty
-    int inner;       // emitted transitions strictly inside (not at the first active sample)
-    int lastL;       // last LOW sample, -1 if none
-    int firstH;      // first HIGH-class sample, INT_MAX if none
-    int lastS;       // last LOW-run start strictly inside, -1 if none
-    int pad0, pad1;
-};
-struct WarpRec {
-    double dsum;     // sum of admitted (x - prev), exact
-    float absd;      // sum of admitted |x - prev| (bounds how far ss can move inside the tile)
-    unsigned flags;  // 1 = some sample was not robustly classifiable
-};
-
-template <int NT, int R>
+template <int NT>
 struct BlockShared {
     static const int NW = NT / 32;
     double wsum[2][NW];
@@ -197,9 +180,6 @@ struct BlockShared {
     unsigned flags[3];
     int emin, emax;
     double red[NW];
-    RowRec rows[2][R * NW];
-    WarpRec warps[2][NW];
-    double rsum[R * NW];  // per-record sums for the band refinement
 };
 
 // everything a segment carries from tile to tile (identical in all threads of the CTA)
@@ -268,13 +248,13 @@ __device__ __forceinline__ void exp_track(float x, int &emin, int &emax) {
 // ---------------------------------------------------------------- exact tile (fix-point over prefix sums)
 // One tile of NT*K samples starting at stream index P0, classes decided with every sample's own exact ss.
 // Always correct (inside the exactly-summable regime); several block barriers per tile.
-template <int NT, int K, int R, bool BM = false>
-__device__ __noinline__ void exact_tile(const SegWork *wp, const SlicerParams *pp, float *ring, BlockShared<NT, R> *shp,
+template <int NT, int K, bool BM = false>
+__device__ __noinline__ void exact_tile(const SegWork *wp, const SlicerParams *pp, float *ring, BlockShared<NT> *shp,
                                         const int64_t P0, const int slot0, SegCarry *cs) {
     constexpr int NW = NT / 32;
     const SegWork &w = *wp;
     const SlicerParams &p = *pp;
-    BlockShared<NT, R> &sh = *shp;
+    BlockShared<NT> &sh = *shp;
     const int L = p.L, mx = p.mx;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t p0 = P0 + (int64_t)tid * K;
@@ -558,19 +538,15 @@ __device__ __noinline__ void exact_tile(const SegWork *wp, const SlicerParams *p
 }
 
 // ---------------------------------------------------------------- the segment kernel
-// A tile is R rows of NT*4 samples.  Fast path (one block barrier per tile): every sample is classified in
-// float against thresholds widened by a guard band that covers any ss the tile can reach; the band is
-// justified afterwards by the block sum of admitted |x - prev|.  Tiles where a sample falls inside the band,
-// the sum exceeds the band, or a HIGH sample follows a LOW sample closely (hysteresis) are redone exactly.
-template <int NT, int K, int R>
-__global__ void __launch_bounds__(NT, (K == 4 ? 4 : 2)) slicer_kernel(const SegWork *__restrict__ works,
-                                                                      const SlicerParams *__restrict__ params) {
-    constexpr int SUB = NT * K;      // samples per row
-    constexpr int T = SUB * R;       // samples per tile
+// First-generation kernel, for the windows the streaming kernel does not take (below 1024 samples or not a multiple of 4):
+// one CTA walks one time segment in tiles of SLICER_NT samples, one sample per thread, each through exact_tile.
+constexpr int SLICER_NT = 256;
+__global__ void __launch_bounds__(SLICER_NT, 2) slicer_kernel(const SegWork *__restrict__ works,
+                                                             const SlicerParams *__restrict__ params) {
+    constexpr int NT = SLICER_NT, T = SLICER_NT;
     constexpr int NW = NT / 32;
-    static_assert(R * NW <= 32, "one lane per row record");
     extern __shared__ __align__(16) float ring[];
-    __shared__ BlockShared<NT, R> sh;
+    __shared__ BlockShared<NT> sh;
 
     // the work item and the parameters live in shared memory: one copy per CTA, no registers held
     __shared__ SegWork w_s;
@@ -583,7 +559,7 @@ __global__ void __launch_bounds__(NT, (K == 4 ? 4 : 2)) slicer_kernel(const SegW
     __syncthreads();
     const SegWork &w = w_s;
     const SlicerParams &p = p_s;
-    const int L = p.L, mx = p.mx;
+    const int L = p.L;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
     // ---- entry state
@@ -633,16 +609,11 @@ __global__ void __launch_bounds__(NT, (K == 4 ? 4 : 2)) slicer_kernel(const SegW
     c.scan_buf = 0;
     c.cnt_buf = 0;
     c.round_no = 0;
-
-    const bool fast_ok = (K == 4) && ((L & 3) == 0) && p.lo > 0.0 && p.hi > p.lo;
-    const bool end_barrier = 2 * T > L;  // a tile would read ring slots the previous tile wrote
-    float absd_prev = 0.0f, absd_prev2 = 0.0f;  // admitted |x - prev| of the last two tiles: size the next guard band
-    double tot_prev = 0.0;               // window-sum change over the previous tile: predicts the drift inside this one
-    unsigned tile_no = 0, n_fast = 0, n_slow = 0, n_refined = 0, n_st2 = 0, n_refbad = 0;
+    unsigned n_exact = 0;
 
     const int64_t tile_first = w.warm_begin / T;
     const int64_t tile_last = (w.end > w.warm_begin) ? (w.end - 1) / T : tile_first - 1;
-    int slot0 = (int)((tile_first * T + (int64_t)tid * K) % L);
+    int slot0 = (int)((tile_first * T + (int64_t)tid) % L);
 
     for (int64_t tile = tile_first; tile <= tile_last; tile++) {
         const int64_t P0 = tile * T;
@@ -673,433 +644,11 @@ __global__ void __launch_bounds__(NT, (K == 4 ? 4 : 2)) slicer_kernel(const SegW
             }
         }
 
-        bool done = false;
-        // interior tile: every sample is inside the segment and the input buffer, and either all or none of
-        // its transitions are written (anything else goes to the exact path, which masks per sample)
-        const bool interior = P0 >= w.warm_begin && P0 + T <= w.end && P0 >= w.in_begin && P0 + T <= w.in_end &&
-                              (P0 >= w.begin || P0 + T <= w.begin);
-        if (fast_ok && interior && c.ss0 > 0.0) {
-            // ---------------------------------------------------------------- fast path
-            const bool emit = P0 >= w.begin;
-            // guard band: ss stays within ss0 +- Dg inside the tile (verified after the barrier)
-            const float Dg = fmaxf(2.0f * fmaxf(absd_prev, absd_prev2), (float)(c.ss0 * 0x1p-14));
-            const double tl = c.ss0 * p.loL, th = c.ss0 * p.hiL;
-            float A1, A2, B1, B2;
-            {
-                const double g = (double)Dg / c.ss0 + 0x1p-20;
-                A1 = __double2float_rd(tl * (1.0 - g)); A2 = __double2float_ru(tl * (1.0 + g));
-                B1 = __double2float_rd(th * (1.0 - g)); B2 = __double2float_ru(th * (1.0 + g));
-            }
-            // the guess for samples inside a band uses the ss predicted for each row from the previous tile's drift
-            const double drift_row = tot_prev * (1.0 / R);
-
-            float x[R * 4];
-            unsigned clsbits = 0u;  // 2 bits per sample: 0 LOW, 1 MID, 2 HIGH
-            unsigned uncbits = 0u;  // 1 bit per sample: inside a guard band (class not proven yet); filled on demand
-            bool any_unc = false;   // some sample of this thread is inside a band
-            const int kind = p.input_kind;
-            const bool f32in = kind == IN_ENVELOPE_F32 || kind == IN_REAL_F32;
-            // ---- phase 0: loads (all rows in flight at once; next tile requested into L2), guessed classes
-            {
-                const char *rowp = reinterpret_cast<const char *>(w.in) + (P0 - w.in_pos0 + (int64_t)tid * 4) * (int64_t)item_size(kind);
-                if (f32in) {
-                    float4 xin[R];
-#pragma unroll
-                    for (int r = 0; r < R; r++) xin[r] = ldg_stream4(reinterpret_cast<const float4 *>(rowp + (size_t)r * SUB * 4));
-                    if (tid < T / 32 && P0 + 2 * T <= w.in_end)
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(rowp + (size_t)T * 4 + (size_t)tid * 112));
-#pragma unroll
-                    for (int r = 0; r < R; r++) {
-                        x[r * 4 + 0] = xin[r].x; x[r * 4 + 1] = xin[r].y; x[r * 4 + 2] = xin[r].z; x[r * 4 + 3] = xin[r].w;
-                    }
-                    if (kind == IN_REAL_F32) {
-#pragma unroll
-                        for (int k = 0; k < R * 4; k++) x[k] = env_real(x[k]);
-                    }
-                } else if (kind == IN_IQ_F32) {
-#pragma unroll
-                    for (int r = 0; r < R; r++) {
-                        const float4 *q = reinterpret_cast<const float4 *>(rowp + (size_t)r * SUB * 8);
-                        const float4 a = ldg_stream4(q), b = ldg_stream4(q + 1);
-                        x[r * 4 + 0] = env_iq(a.x, a.y); x[r * 4 + 1] = env_iq(a.z, a.w);
-                        x[r * 4 + 2] = env_iq(b.x, b.y); x[r * 4 + 3] = env_iq(b.z, b.w);
-                    }
-                } else {
-#pragma unroll
-                    for (int r = 0; r < R; r++) {
-                        const short4 sv = __ldg(reinterpret_cast<const short4 *>(rowp + (size_t)r * SUB * 2));
-                        x[r * 4 + 0] = env_real(__fdiv_rn((float)sv.x, p.pcm_scale));
-                        x[r * 4 + 1] = env_real(__fdiv_rn((float)sv.y, p.pcm_scale));
-                        x[r * 4 + 2] = env_real(__fdiv_rn((float)sv.z, p.pcm_scale));
-                        x[r * 4 + 3] = env_real(__fdiv_rn((float)sv.w, p.pcm_scale));
-                    }
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < R; r++) {
-                const double ssp = c.ss0 + ((double)r + 0.5) * drift_row;
-                // a robust sample must get its proven class: clamp the guess thresholds into the bands
-                const float TL = fminf(fmaxf(__double2float_rn(ssp * p.loL), A1), A2);
-                const float TH = fminf(fmaxf(__double2float_rn(ssp * p.hiL), B1), B2);
-#pragma unroll
-                for (int j = 0; j < 4; j++) {
-                    const float xv = x[r * 4 + j];
-                    const unsigned code = 1u + (xv > TH ? 1u : 0u) - (xv < TL ? 1u : 0u);
-                    clsbits |= code << (2 * (r * 4 + j));
-                    any_unc = any_unc || ((xv >= A1) && (xv <= A2)) || ((xv >= B1) && (xv <= B2));
-                }
-            }
-            if (__any_sync(FULL, any_unc)) {  // rare: remember which samples
-#pragma unroll
-                for (int k = 0; k < R * 4; k++) {
-                    const float xv = x[k];
-                    const bool inband = ((xv >= A1) && (xv <= A2)) || ((xv >= B1) && (xv <= B2));
-                    uncbits |= (inband ? 1u : 0u) << k;
-                }
-            }
-
-            bool slow = false;
-            double tot = 0.0;
-            float absD = 0.0f;
-            int tot_tr = 0, cnt = 0, basecnt = 0, prevlast = 0, tile_last_val = 3, first_val = 3, first_pos = 0;
-            bool btrans = false;
-            RowRec rec;
-            for (int iter = 0;; iter++, tile_no++) {
-                const int buf = tile_no & 1;
-                // ---- phase 1: sums of the admitted deltas and the row records, from the current classes
-                double dsum = 0.0;
-                float absd = 0.0f;
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    int s0 = slot0 + r * SUB;
-                    if (s0 >= L) s0 -= L;
-                    const float4 pv4 = *reinterpret_cast<const float4 *>(ring + s0);
-                    const float prev[4] = {pv4.x, pv4.y, pv4.z, pv4.w};
-                    const unsigned codes = (clsbits >> (8 * r)) & 0xffu;
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        if (((codes >> (2 * j)) & 3u) == 1u) {  // MID: admitted
-                            dsum += (double)x[r * 4 + j] - (double)prev[j];
-                            absd += fabsf(x[r * 4 + j] - prev[j]);
-                        }
-                    }
-                    // row record of this warp (128 samples): per-thread edges, warp reductions
-                    RowRec rr;
-                    const int base = r * SUB + warp * 128;  // sample (lane, j) sits at base + 4*lane + j
-                    rr.first = (base << 2) | 1; rr.last = ((base + 127) << 2) | 1;
-                    rr.inner = 0; rr.lastL = -1; rr.firstH = INT_MAX; rr.lastS = -1; rr.pad0 = rr.pad1 = 0;
-                    if (__any_sync(FULL, codes != 0x55u)) {  // something other than MID in these 128 samples
-                        const unsigned c3 = (codes >> 6) & 3u;
-                        unsigned pc = __shfl_up_sync(FULL, c3, 1);      // previous sample's class for j = 0
-                        const unsigned lastc = __shfl_sync(FULL, c3, 31);
-                        const unsigned firstc = __shfl_sync(FULL, codes & 3u, 0);
-                        if (lane == 0) pc = codes & 3u;                  // the record's first sample is not "inside"
-                        // class of the previous sample for each j, packed like `codes`
-                        const unsigned prevs = ((codes << 2) | pc) & 0xffu;
-                        const unsigned diff = codes ^ prevs;             // non-zero 2-bit field = transition
-                        const unsigned tr = (diff | (diff >> 1)) & 0x55u;
-                        const unsigned isL = ~(codes | (codes >> 1)) & 0x55u;   // field == 0
-                        const unsigned isH = (codes >> 1) & 0x55u;              // field == 2
-                        const unsigned pL = ~(prevs | (prevs >> 1)) & 0x55u;
-                        if (emit) rr.inner = __reduce_add_sync(FULL, __popc(tr));
-                        const int pos0 = base + 4 * lane;
-                        // highest j with LOW / lowest j with HIGH / highest j where a LOW run starts (bit 2j -> j)
-                        const int myL = isL ? pos0 + ((31 - __clz(isL)) >> 1) : -1;
-                        const int myH = isH ? pos0 + ((__ffs(isH) - 1) >> 1) : INT_MAX;
-                        const unsigned st = isL & ~pL & (lane == 0 ? ~1u : ~0u);
-                        const int myS = st ? pos0 + ((31 - __clz(st)) >> 1) : -1;
-                        rr.lastL = __reduce_max_sync(FULL, myL);
-                        rr.firstH = __reduce_min_sync(FULL, myH);
-                        rr.lastS = __reduce_max_sync(FULL, myS);
-                        rr.first = (base << 2) | (int)firstc;
-                        rr.last = ((base + 127) << 2) | (int)lastc;
-                    }
-                    if (lane == 0) sh.rows[buf][r * NW + warp] = rr;
-                }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    dsum += __shfl_xor_sync(FULL, dsum, o);
-                    absd += __shfl_xor_sync(FULL, absd, o);
-                }
-                const unsigned uncertain = __any_sync(FULL, uncbits != 0u) ? 1u : 0u;
-                if (lane == 0) {
-                    WarpRec wr;
-                    wr.dsum = dsum; wr.absd = absd; wr.flags = uncertain;
-                    sh.warps[buf][warp] = wr;
-                }
-                __syncthreads();  // the only barrier of a tile whose samples are all outside the bands
-
-                // ---- phase 2: every warp scans the records redundantly: lane l <-> record l (row-major = stream order)
-                tot = 0.0;
-                absD = 0.0f;
-                unsigned unc = 0u;
-                if (lane < NW) {
-                    const WarpRec wr = sh.warps[buf][lane];
-                    tot = wr.dsum; absD = wr.absd; unc = wr.flags;
-                }
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) {
-                    tot += __shfl_xor_sync(FULL, tot, o);
-                    absD += __shfl_xor_sync(FULL, absD, o);
-                }
-                unc = __any_sync(FULL, unc != 0u) ? 1u : 0u;
-                rec.first = INT_MAX; rec.last = -1; rec.inner = 0; rec.lastL = -1; rec.firstH = INT_MAX; rec.lastS = -1;
-                if (lane < R * NW) rec = sh.rows[buf][lane];
-                const bool has = rec.last >= 0;
-                // last defined val before each record (exclusive), seeded with the carry
-                int ld = has ? (rec.last & 3) - 1 : 3;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int n = __shfl_up_sync(FULL, ld, o);
-                    if (lane >= o && ld == 3) ld = n;
-                }
-                prevlast = __shfl_up_sync(FULL, ld, 1);
-                if (lane == 0 || prevlast == 3) prevlast = c.last_val;
-                tile_last_val = __shfl_sync(FULL, ld, 31);
-                // running maximum of the last LOW position before each record (exclusive), seeded with the carry
-                const int64_t cl = c.lastL == NO_POS ? (int64_t)INT_MIN / 2 : c.lastL - P0;
-                const int carryL = (int)max(cl, (int64_t)INT_MIN / 2);
-                int mxL = rec.lastL >= 0 ? rec.lastL : INT_MIN / 2;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int n = __shfl_up_sync(FULL, mxL, o);
-                    if (lane >= o) mxL = max(mxL, n);
-                }
-                int exL = __shfl_up_sync(FULL, mxL, 1);
-                if (lane == 0) exL = INT_MIN / 2;
-                exL = max(exL, carryL);
-                const bool hasH = rec.firstH != INT_MAX;
-                // hysteresis can matter only if a HIGH sample comes within max_len + 1 samples after a LOW sample
-                const bool st2_risk = hasH && ((rec.lastL >= 0) || ((int64_t)rec.firstH - (int64_t)exL <= (int64_t)mx + 1));
-                first_val = has ? (rec.first & 3) - 1 : 3;
-                first_pos = has ? (rec.first >> 2) : 0;
-                btrans = has && first_val != prevlast;
-                cnt = rec.inner + ((btrans && emit) ? 1 : 0);
-                int inc = cnt;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const int n = __shfl_up_sync(FULL, inc, o);
-                    if (lane >= o) inc += n;
-                }
-                tot_tr = __shfl_sync(FULL, inc, 31);
-                basecnt = inc - cnt;
-                if (__any_sync(FULL, st2_risk)) {
-                    n_st2++;
-                    slow = true;
-                    break;
-                }
-                if (!(absD * 1.001f <= Dg) || iter > 0) {
-                    // the window sum moved further than the band assumed (or classes were just corrected): size the
-                    // band from what was measured and re-mark the samples inside it
-                    const double gw = (double)(fmaxf(absD, Dg) * 1.001f) / c.ss0 + 0x1p-20;
-                    A1 = __double2float_rd(tl * (1.0 - gw)); A2 = __double2float_ru(tl * (1.0 + gw));
-                    B1 = __double2float_rd(th * (1.0 - gw)); B2 = __double2float_ru(th * (1.0 + gw));
-                    if (iter == 0) {
-                        uncbits = 0u;
-#pragma unroll
-                        for (int k = 0; k < R * 4; k++) {
-                            const float xv = x[k];
-                            const bool inband = ((xv >= A1) && (xv <= A2)) || ((xv >= B1) && (xv <= B2));
-                            uncbits |= (inband ? 1u : 0u) << k;
-                        }
-                        unc = 1u;  // block-uniform: take the refinement path, which votes
-                    }
-                }
-                if (!unc) break;  // every class is proven
-
-                // ---- refinement: samples inside the tile-wide band.  First against the band of their own 128-sample
-                // record, whose start ss is exact given the current classes; what even that cannot decide gets its
-                // own exact ss (prefix inside the record) and the exact ratio test.  A sample whose exact class
-                // differs from the current one is corrected and the tile goes round again (self-consistency).
-                float rabs[R];
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    int s0 = slot0 + r * SUB;
-                    if (s0 >= L) s0 -= L;
-                    const float4 pv4 = *reinterpret_cast<const float4 *>(ring + s0);
-                    const float prev[4] = {pv4.x, pv4.y, pv4.z, pv4.w};
-                    double ds = 0.0;
-                    float da = 0.0f;
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        if (((clsbits >> (2 * (r * 4 + j))) & 3u) == 1u) {
-                            ds += (double)x[r * 4 + j] - (double)prev[j];
-                            da += fabsf(x[r * 4 + j] - prev[j]);
-                        }
-                    }
-#pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) {
-                        ds += __shfl_xor_sync(FULL, ds, o);
-                        da += __shfl_xor_sync(FULL, da, o);
-                    }
-                    rabs[r] = da;
-                    if (lane == 0) sh.rsum[r * NW + warp] = ds;
-                }
-                __syncthreads();
-                double pre = (lane < R * NW) ? sh.rsum[lane] : 0.0;
-                const double own = pre;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) {
-                    const double n = __shfl_up_sync(FULL, pre, o);
-                    if (lane >= o) pre += n;
-                }
-                pre -= own;  // exclusive: sum of the records before record `lane`
-                unsigned flipped = 0u, bad = 0u;
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    const int q = r * NW + warp;
-                    const double ssq = c.ss0 + __shfl_sync(FULL, pre, q);
-                    unsigned resid = 0u;
-                    if (((uncbits >> (4 * r)) & 15u) != 0u) {
-                        if (!(ssq > 0.0)) bad = 1u;
-                        const double g2 = (double)(rabs[r] * 1.001f) / ssq + 0x1p-20;
-                        const double tl2 = ssq * p.loL, th2 = ssq * p.hiL;
-                        const float a1 = __double2float_rd(tl2 * (1.0 - g2)), a2 = __double2float_ru(tl2 * (1.0 + g2));
-                        const float b1 = __double2float_rd(th2 * (1.0 - g2)), b2 = __double2float_ru(th2 * (1.0 + g2));
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            if ((uncbits >> (4 * r + j)) & 1u) {
-                                const float xv = x[r * 4 + j];
-                                const unsigned code = (clsbits >> (2 * (r * 4 + j))) & 3u;
-                                // does the current class hold for every ss the record can reach?
-                                const bool ok = code == 0u ? (xv < a1) : (code == 2u ? (xv > a2 && xv > b2) : (xv > a2 && xv < b1));
-                                if (!ok) resid |= 1u << j;
-                            }
-                        }
-                    }
-                    if (__any_sync(FULL, resid != 0u)) {  // warp-uniform
-                        int s0 = slot0 + r * SUB;
-                        if (s0 >= L) s0 -= L;
-                        const float4 pv4 = *reinterpret_cast<const float4 *>(ring + s0);
-                        const float prev[4] = {pv4.x, pv4.y, pv4.z, pv4.w};
-                        double pre4[4];
-                        double run = 0.0;
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            pre4[j] = run;
-                            if (((clsbits >> (2 * (r * 4 + j))) & 3u) == 1u) run += (double)x[r * 4 + j] - (double)prev[j];
-                        }
-                        double incl = run;
-#pragma unroll
-                        for (int o = 1; o < 32; o <<= 1) {
-                            const double n = __shfl_up_sync(FULL, incl, o);
-                            if (lane >= o) incl += n;
-                        }
-                        const double lane_base = ssq + (incl - run);
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            if (resid & (1u << j)) {
-                                const unsigned cc = (unsigned)(classify(x[r * 4 + j], lane_base + pre4[j], p) + 1);
-                                const int sh2 = 2 * (r * 4 + j);
-                                if (cc != ((clsbits >> sh2) & 3u)) {
-                                    clsbits = (clsbits & ~(3u << sh2)) | (cc << sh2);  // corrected; verified again next round
-                                    flipped = 1u;
-                                }
-                            }
-                        }
-                    }
-                }
-                const int vote = __syncthreads_or((int)(flipped | (bad << 1)));
-                if (vote == 0) {  // every sample inside the bands has been verified against its exact ss
-                    n_refined++;
-                    break;
-                }
-                if (__syncthreads_or((int)bad) || iter >= 3) {
-                    n_refbad++;
-                    slow = true;
-                    break;
-                }
-            }
-            tile_no++;
-            absd_prev2 = absd_prev;
-            absd_prev = absD;  // sizes the next tiles' band
-            if (!slow) {
-                done = true;
-                // admitted samples lie strictly between the LOW and HIGH bands: exponent range from the thresholds
-                exp_track(A1, emin, emax);
-                exp_track(B2, emin, emax);
-                // ---- ring update and transitions, row by row
-#pragma unroll
-                for (int r = 0; r < R; r++) {
-                    int s0 = slot0 + r * SUB;
-                    if (s0 >= L) s0 -= L;
-                    const unsigned codes = (clsbits >> (8 * r)) & 0xffu;
-                    if (codes == 0x55u) {
-                        *reinterpret_cast<float4 *>(ring + s0) = make_float4(x[r * 4], x[r * 4 + 1], x[r * 4 + 2], x[r * 4 + 3]);
-                    } else {
-                        float4 pv4 = *reinterpret_cast<const float4 *>(ring + s0);
-                        if (((codes >> 0) & 3u) == 1u) pv4.x = x[r * 4 + 0];
-                        if (((codes >> 2) & 3u) == 1u) pv4.y = x[r * 4 + 1];
-                        if (((codes >> 4) & 3u) == 1u) pv4.z = x[r * 4 + 2];
-                        if (((codes >> 6) & 3u) == 1u) pv4.w = x[r * 4 + 3];
-                        *reinterpret_cast<float4 *>(ring + s0) = pv4;
-                    }
-                    const int q = r * NW + warp;
-                    const int rcnt = __shfl_sync(FULL, cnt, q);
-                    if (rcnt > 0) {  // warp-uniform
-                        const int rbase = __shfl_sync(FULL, basecnt, q);
-                        const int rprev = __shfl_sync(FULL, prevlast, q);
-                        const int v3 = (int)((codes >> 6) & 3u) - 1;
-                        int prevv = __shfl_up_sync(FULL, v3, 1);
-                        if (lane == 0) prevv = rprev;
-                        unsigned trm = 0u;
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            const int v = (int)((codes >> (2 * j)) & 3u) - 1;
-                            if (v != prevv) trm |= 1u << j;
-                            prevv = v;
-                        }
-                        const int mine = __popc(trm);
-                        int pre = mine;
-#pragma unroll
-                        for (int o = 1; o < 32; o <<= 1) {
-                            const int n = __shfl_up_sync(FULL, pre, o);
-                            if (lane >= o) pre += n;
-                        }
-                        uint32_t idx = c.seg_count + (uint32_t)rbase + (uint32_t)(pre - mine);
-                        const uint32_t rel = (uint32_t)(P0 + (int64_t)r * SUB + (int64_t)tid * 4 - w.slab_pos0);
-#pragma unroll
-                        for (int j = 0; j < 4; j++) {
-                            if (trm & (1u << j)) {
-                                if (idx < w.trans_cap) w.trans[idx] = pack_trans(rel + j, (int)((codes >> (2 * j)) & 3u) - 1);
-                                idx++;
-                            }
-                        }
-                    }
-                }
-                // ---- carries
-                c.seg_count += (uint32_t)tot_tr;
-                c.ss0 += tot;
-                tot_prev = tot;
-                if (tile_last_val != 3) c.last_val = tile_last_val;
-                const int newL = __reduce_max_sync(FULL, rec.lastL);
-                if (newL >= 0) {
-                    int sc = rec.lastS;
-                    if (btrans && first_val == -1) sc = max(sc, first_pos);
-                    const int newS = __reduce_max_sync(FULL, sc);
-                    c.lastL = P0 + newL;
-                    if (newS >= 0) c.lrun_start = P0 + newS;
-                }
-                n_fast++;
-                if (end_barrier) __syncthreads();
-            }
-        }
-        if (!done) {
-            // ---------------------------------------------------------------- exact path, row by row
-            if (tid == 0) c_s = c;
-            __syncthreads();
-#pragma unroll 1
-            for (int r = 0; r < R; r++) {
-                const int64_t Pr = P0 + (int64_t)r * SUB;
-                if (Pr >= w.end || Pr + SUB <= w.warm_begin) continue;  // block-uniform
-                int s0 = slot0 + r * SUB;
-                if (s0 >= L) s0 -= L;
-                exact_tile<NT, K, R>(&w_s, &p_s, ring, &sh, Pr, s0, &c_s);
-            }
-            tot_prev = c_s.ss0 - c.ss0;
-            c = c_s;
-            n_slow++;
-        }
+        if (tid == 0) c_s = c;
+        __syncthreads();
+        exact_tile<NT, 1>(&w_s, &p_s, ring, &sh, P0, slot0, &c_s);
+        c = c_s;
+        n_exact++;
         slot0 += T % L;
         if (slot0 >= L) slot0 -= L;
     }
@@ -1131,12 +680,8 @@ __global__ void __launch_bounds__(NT, (K == 4 ? 4 : 2)) slicer_kernel(const SegW
     if (tid == 0 && w.trans_count) *w.trans_count = c.seg_count;
     if (tid == 0 && w.status) *w.status = status;
     if (tid == 0) {
-        atomicAdd(&g_tile_stats[0], (unsigned long long)n_fast);
-        atomicAdd(&g_tile_stats[1], (unsigned long long)n_slow);
+        atomicAdd(&g_tile_stats[1], (unsigned long long)n_exact);
         atomicAdd(&g_tile_stats[8], (unsigned long long)c.round_no);
-        atomicAdd(&g_tile_stats[9], (unsigned long long)n_refined);
-        atomicAdd(&g_tile_stats[6], (unsigned long long)n_st2);
-        atomicAdd(&g_tile_stats[10], (unsigned long long)n_refbad);
     }
 }
 
@@ -1281,26 +826,15 @@ __global__ void seam_compare_kernel(const SlicerHdr *const *__restrict__ truth, 
 }
 
 // ---------------------------------------------------------------- host launchers
-// rows per tile of the vector kernel for a given window: a tile must fit twice into the ring
-int slicer_rows(int L) { return L >= 8192 ? 4 : (L >= 4096 ? 2 : 1); }
-bool slicer_streaming_ok(int L, bool vec_ok);
+bool slicer_streaming_ok(int L, int kind);
 int slicer_streaming_tile(int L, int kind);
 // tile of the kernel a window takes: segment boundaries and halos are whole tiles
-int slicer_tile(int L, bool vec_ok, int kind) {
-    if (slicer_streaming_ok(L, vec_ok)) return slicer_streaming_tile(L, kind);
-    return (vec_ok && L >= 1024) ? 1024 * slicer_rows(L) : 256;
+int slicer_tile(int L, int kind) {
+    if (slicer_streaming_ok(L, kind)) return slicer_streaming_tile(L, kind);
+    return SLICER_NT;
 }
 
 static int raise_dynamic_smem(const void *fn, size_t smem);
-
-template <int NT, int K, int R>
-static int launch_one(const SegWork *d_works, int n_works, const SlicerParams *d_params, size_t smem, cudaStream_t stream) {
-    auto k = slicer_kernel<NT, K, R>;
-    if (raise_dynamic_smem((const void *)k, smem)) return -1;
-    k<<<n_works, NT, smem, stream>>>(d_works, d_params);
-    NFC_CUDA_CHECK(cudaGetLastError());
-    return 0;
-}
 
 // ---- variants of the streaming kernel.  Default: the pipelined one (slicer_pipe.cuh), two CTAs of 8 + 2 warps per SM with
 // three stages of 4096 samples (NFC_SLICER_STAGES=2: two); windows too long for that (20 MS/s: 80 KB ring) take 16 + 2 warps,
@@ -1408,13 +942,14 @@ static int raise_dynamic_smem(const void *fn, size_t smem) {
     return 0;
 }
 
-// the streaming kernel needs two tiles of 4096 samples to fit into the window (and the window, a tile and the kernel's
-// own scratch into one CTA's shared memory); NFC_SLICER_OLD=1 keeps the first-generation kernel
-bool slicer_streaming_ok(int L, bool vec_ok) {
-    static const bool old = getenv("NFC_SLICER_OLD") && getenv("NFC_SLICER_OLD")[0] == '1';
-    static const bool no_small = getenv("NFC_SLICER_SMALL") && getenv("NFC_SLICER_SMALL")[0] == '0';
-    if (!(vec_ok && L >= (no_small ? FAST_BIG_MIN_L : FAST_SMALL_MIN_L) && !old)) return false;
-    return fast_variant_of(L, IN_IQ_F32).smem + 16384 + FAST_STATIC_SMEM <= smem_optin_limit();
+// the streaming kernel takes windows that are a multiple of 4 from 1024 samples on, as long as the variant chosen for the
+// window fits one CTA's shared memory: its dynamic part (ring and staging) and the kernel's static scratch
+bool slicer_streaming_ok(int L, int kind) {
+    if (L % 4 != 0 || L < FAST_SMALL_MIN_L) return false;
+    const FastVariant v = fast_variant_of(L, kind);
+    cudaFuncAttributes fa;
+    if (cudaFuncGetAttributes(&fa, v.fn) != cudaSuccess) return false;
+    return v.smem + fa.sharedSizeBytes <= smem_optin_limit();
 }
 
 static int apply_pipe_tuning() {
@@ -1445,18 +980,13 @@ int launch_slicer_streaming(const SegWork *d_works, int n_works, const SlicerPar
     return 0;
 }
 
-int launch_slicer(const SegWork *d_works, int n_works, const SlicerParams *d_params, int L, bool vec_ok,
-                  cudaStream_t stream) {
+int launch_slicer(const SegWork *d_works, int n_works, const SlicerParams *d_params, int L, cudaStream_t stream) {
     if (n_works <= 0) return 0;
     const size_t smem = ((size_t)L * 4 + 15) / 16 * 16;
-    if (vec_ok && L >= 1024) {
-        switch (slicer_rows(L)) {
-            case 4: return launch_one<256, 4, 4>(d_works, n_works, d_params, smem, stream);
-            case 2: return launch_one<256, 4, 2>(d_works, n_works, d_params, smem, stream);
-            default: return launch_one<256, 4, 1>(d_works, n_works, d_params, smem, stream);
-        }
-    }
-    return launch_one<256, 1, 1>(d_works, n_works, d_params, smem, stream);
+    if (raise_dynamic_smem((const void *)slicer_kernel, smem)) return -1;
+    slicer_kernel<<<n_works, SLICER_NT, smem, stream>>>(d_works, d_params);
+    NFC_CUDA_CHECK(cudaGetLastError());
+    return 0;
 }
 
 int slicer_tile_stats(unsigned long long *out4, bool reset) {
@@ -1481,28 +1011,19 @@ int slicer_tile_stats(unsigned long long *out4, bool reset) {
 }
 
 // CTAs of the slicer kernel that fit on the device at once (for sizing the number of segments)
-int slicer_resident_ctas(int L, bool vec_ok, int kind) {
+int slicer_resident_ctas(int L, int kind) {
     int dev = 0, sms = 0, per = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const size_t smem = ((size_t)L * 4 + 15) / 16 * 16;
     cudaError_t e = cudaSuccess;
-    const void *fn;
-    int threads = 256;
-    size_t dyn = smem;
-    if (slicer_streaming_ok(L, vec_ok)) {
+    const void *fn = (const void *)slicer_kernel;
+    int threads = SLICER_NT;
+    size_t dyn = ((size_t)L * 4 + 15) / 16 * 16;
+    if (slicer_streaming_ok(L, kind)) {
         const FastVariant v = fast_variant_of(L, kind);
         fn = v.fn;
         threads = v.threads;
         dyn = v.smem;
-    } else if (vec_ok && L >= 1024) {
-        switch (slicer_rows(L)) {
-            case 4: fn = (const void *)slicer_kernel<256, 4, 4>; break;
-            case 2: fn = (const void *)slicer_kernel<256, 4, 2>; break;
-            default: fn = (const void *)slicer_kernel<256, 4, 1>;
-        }
-    } else {
-        fn = (const void *)slicer_kernel<256, 1, 1>;
     }
     if (raise_dynamic_smem(fn, dyn) == 0) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, fn, threads, dyn);
     if (e != cudaSuccess || per < 1) per = 1;

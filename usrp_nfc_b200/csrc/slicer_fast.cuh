@@ -350,7 +350,7 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
     constexpr int BM_WARPS = NW - BM_FIRST;
     constexpr int CARRY_THREAD = NT >= 256 ? 128 : 96;  // not in warp 0: that one has the longest way to the next barrier already
     extern __shared__ __align__(16) float ring[];
-    __shared__ BlockShared<NT, 1> sh;  // exact_tile's scratch
+    __shared__ BlockShared<NT> sh;  // exact_tile's scratch
     __shared__ FastShared<NT, R> fs;
     __shared__ SegWork w_s;
     __shared__ SlicerParams p_s;
@@ -1173,7 +1173,7 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
                 if (Pr >= w.end || Pr + SUB <= w.warm_begin) continue;  // block-uniform
                 int s0 = slot_x + r * SUB;
                 while (s0 >= L) s0 -= L;
-                exact_tile<NT, 4, 1, true>(&w_s, &p_s, ring, &sh, Pr, s0, &c_s);
+                exact_tile<NT, 4, true>(&w_s, &p_s, ring, &sh, Pr, s0, &c_s);
             }
             if (warp == 0) {
                 const double ss1 = c_s.ss0;

@@ -25,8 +25,8 @@
 namespace nfc {
 
 // ---- launchers implemented in the kernel files
-int launch_slicer(const SegWork *d_works, int n_works, const SlicerParams *d_params, int L, bool vec_ok, cudaStream_t);
-bool slicer_streaming_ok(int L, bool vec_ok);
+int launch_slicer(const SegWork *d_works, int n_works, const SlicerParams *d_params, int L, cudaStream_t);
+bool slicer_streaming_ok(int L, int kind);
 int launch_slicer_streaming(const SegWork *d_works, int n_works, const SlicerParams *d_params, int L, int kind, cudaStream_t);
 int launch_extract_count(const uint32_t *d_bm, int64_t bm_pos0, int64_t a, int64_t b, const RunCarry *d_rc_in, int carry_from_bm,
                          uint32_t *d_block_counts, uint32_t *d_block_offsets, uint32_t *d_scan_scratch, uint32_t *d_total,
@@ -65,8 +65,8 @@ int launch_linecode_write(const EventRec *d_ev, const uint32_t *d_M, uint32_t ca
                           uint8_t *d_bits1, uint32_t cap_b1, void *d_frames, void *d_findex, uint32_t cap_em, int64_t a,
                           const void *d_bits_in, void *d_bits_out, uint32_t *d_n_empty, uint32_t *d_n_frames, const uint32_t *d_pending_in,
                           const DecCarry *d_carry_in, DecCarry *d_carry_out, uint32_t *d_pending_out, cudaStream_t stream);
-int slicer_tile(int L, bool vec_ok, int kind);
-int slicer_resident_ctas(int L, bool vec_ok, int kind);
+int slicer_tile(int L, int kind);
+int slicer_resident_ctas(int L, int kind);
 int slicer_tile_stats(unsigned long long *out4, bool reset);
 int launch_batch_warm(const void *d_items, int64_t stride_bytes, int64_t pitch, int n_cap, int L, const SlicerParams *d_params,
                       void *d_states, size_t state_bytes, cudaStream_t stream);
@@ -329,9 +329,10 @@ struct Stream {
 
     nfc_stats stats;
 
-    int tile() const { return slicer_tile(sp.L, vec_ok(), sp.input_kind); }
-    bool vec_ok() const { return (sp.L % 4) == 0; }
-    // (windows whose ring does not fit a CTA's shared memory beside the kernels' own scratch take the sequential kernel)
+    int tile() const { return slicer_tile(sp.L, sp.input_kind); }
+    // windows of 256 to 52000 samples take the streaming kernel (multiples of 4 from 1024 on) or the first-generation kernel;
+    // the others take the sequential kernel: shorter ones than a tile, and longer ones, whose ring does not fit a CTA's shared
+    // memory beside the kernels' own scratch
     bool parallel_ok() const { return sp.L >= 256 && sp.L <= 52000 && !force_serial && !serial_mode; }
 
     int init(const nfc_params *p);
@@ -364,7 +365,7 @@ struct Stream {
     // the share of the speculative starts; the slabs after the first take their transitions from the bitmap (extract_only)
     int64_t super_slab = 5;
     bool super_balance = true;  // NFC_SUPER_BALANCE=0: every launch but the last takes super_slab slabs
-    bool streaming_ok() const { return parallel_ok() && slicer_streaming_ok(sp.L, vec_ok()); }
+    bool streaming_ok() const { return parallel_ok() && slicer_streaming_ok(sp.L, sp.input_kind); }
 };
 
 int Stream::ensure_pinned(int idx, size_t bytes) {
@@ -472,7 +473,7 @@ int Stream::init(const nfc_params *p) {
 
     warm.reserve((size_t)sp.L);
     if (state.ensure(state_block_bytes(sp.L))) return -1;
-    resident_ctas = parallel_ok() ? slicer_resident_ctas(sp.L, vec_ok(), sp.input_kind) : 1;
+    resident_ctas = parallel_ok() ? slicer_resident_ctas(sp.L, sp.input_kind) : 1;
     if (const char *e = getenv("NFC_SUPER_SLAB")) super_slab = std::max(1, std::min(8, atoi(e)));
     if (const char *e = getenv("NFC_SUPER_BALANCE")) super_balance = atoi(e) != 0;
     return 0;
@@ -695,7 +696,7 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
         return -1;
     }
     if (!streaming_ok()) {
-        set_error("push_batch: needs the streaming slicer (av_window >= 1024, a multiple of 4)");
+        set_error("push_batch: needs the streaming slicer (av_window in [1024, 52000], a multiple of 4)");
         return -1;
     }
     if (n_cap <= 0 || cap_len <= (int64_t)L + 2 * sp.mx || stride_items < cap_len || L <= sp.mx + 1) {
@@ -967,7 +968,7 @@ int Stream::run_slicer(Slicer kind, const void *d_in, int64_t in_pos0, int64_t i
         if (kind == Slicer::streaming) {
             if (launch_streaming(d_works, n_works)) return -1;
         } else if (kind == Slicer::first_gen) {
-            if (launch_slicer(d_works, n_works, params_d.as<SlicerParams>(), L, vec_ok(), cs)) return -1;
+            if (launch_slicer(d_works, n_works, params_d.as<SlicerParams>(), L, cs)) return -1;
         } else {
             if (launch_slicer_serial(d_works, n_works, params_d.as<SlicerParams>(), serial_ring.as<float>(), (size_t)L + 16, cs))
                 return -1;

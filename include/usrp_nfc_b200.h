@@ -27,7 +27,9 @@ enum {
     NFC_IN_ENVELOPE_F32 = 0, /* float32 |z|^2 -- transition_sink's in_sig (transition_sink.py:16)             */
     NFC_IN_REAL_F32 = 1,     /* float32 WAV samples; envelope = x*x on device (decoder.py:25-28)             */
     NFC_IN_IQ_F32 = 2,       /* complex64 from UHD; envelope = re^2+im^2 on device (usrp_src.py:31)          */
-    NFC_IN_PCM_S16 = 3       /* int16 PCM; /pcm_scale, then x*x on device (blocks.wavfile_source, unpinned)  */
+    NFC_IN_PCM_S16 = 3,      /* int16 PCM; /pcm_scale, then x*x on device (blocks.wavfile_source, unpinned)  */
+    NFC_IN_SC16 = 4          /* complex int16 (UHD sc16: I then Q, 4 B); each /pcm_scale, then re^2+im^2 on device,
+                              * exactly as NFC_IN_IQ_F32 for (I/pcm_scale, Q/pcm_scale) (usrp_src.py:31)          */
 };
 enum { NFC_MEM_HOST = 0, NFC_MEM_DEVICE = 1 };
 /* which outputs a stream materialises */
@@ -45,10 +47,10 @@ typedef struct {
     int32_t max_len;   /* 50, in samples   */
     int32_t decode_reader; /* background(reader=...) */
     int32_t decode_tag;    /* background(tag=...)    */
-    int32_t input_kind;    /* NFC_IN_*  */
+    int32_t input_kind;    /* NFC_IN_*; nfc_stream_create rejects any other value */
     int32_t outputs;       /* NFC_OUT_* bit mask; NFC_OUT_DROPPED_EVENTS keeps the type -1 events too */
     int32_t device;        /* CUDA device ordinal */
-    float pcm_scale;       /* divisor for NFC_IN_PCM_S16, 32767 = GNU Radio's 16-bit WAV normalisation */
+    float pcm_scale;       /* divisor for NFC_IN_PCM_S16 and NFC_IN_SC16, 32767 = GNU Radio's 16-bit WAV normalisation */
 } nfc_params;
 
 /* One element of the list handed to transition_sink's callback (transition_sink.py:89-90,97):
@@ -99,8 +101,8 @@ int nfc_stream_set_thresholds(nfc_stream *s, double lo_val, double hi_val);
  * the handle's own CUDA stream: the work that produces them must have completed when the call is made. */
 int64_t nfc_stream_push(nfc_stream *s, const void *items, int64_t n, int mem, int *called_back);
 
-/* A batch of independent captures in one pass: n_captures captures of items_per_capture items each, capture c starting
- * at items + c * stride_items.  In the reference every capture is its own decoder (decoder.py:16-33): its own
+/* A batch of independent captures in one pass: n_captures captures of items_per_capture items each (of the stream's input
+ * kind: an NFC_IN_SC16 capture holds items_per_capture sc16 items, 4 B each), capture c starting at items + c * stride_items.  In the reference every capture is its own decoder (decoder.py:16-33): its own
  * transition_sink with its own warm-up and lo_val / hi_val (transition_sink.py:12-34,109-125; lo_vals / hi_vals: one value
  * per capture, NULL = the stream's), its own background thread, Miller / Manchester decoders and PacketProcessors
  * (background.py:17-25).  The stream must be new or reset; its outputs afterwards are those of all captures, positions

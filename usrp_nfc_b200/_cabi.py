@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # USRP_NFC_B200_LIB: another build of the same library (A/B measurements of kernel variants)
 LIB_PATH = os.environ.get("USRP_NFC_B200_LIB") or os.path.join(_HERE, "libusrp_nfc_b200.so")
 
-IN_ENVELOPE_F32, IN_REAL_F32, IN_IQ_F32, IN_PCM_S16 = 0, 1, 2, 3
+IN_ENVELOPE_F32, IN_REAL_F32, IN_IQ_F32, IN_PCM_S16, IN_SC16 = 0, 1, 2, 3, 4
 MEM_HOST, MEM_DEVICE = 0, 1
 OUT_EVENTS, OUT_SYMBOLS, OUT_FRAMES, OUT_DROPPED_EVENTS = 1, 2, 4, 8
 OUT_ALL = OUT_EVENTS | OUT_SYMBOLS | OUT_FRAMES | OUT_DROPPED_EVENTS
@@ -124,12 +124,38 @@ def last_error():
 
 
 def _torch_dtype_name(input_kind):
-    return {IN_ENVELOPE_F32: "float32", IN_REAL_F32: "float32", IN_IQ_F32: "complex64", IN_PCM_S16: "int16"}[input_kind]
+    return {IN_ENVELOPE_F32: "float32", IN_REAL_F32: "float32", IN_IQ_F32: "complex64", IN_PCM_S16: "int16",
+            IN_SC16: "int16"}[input_kind]
+
+
+def _is_tensor(items):
+    return hasattr(items, "data_ptr") and hasattr(items, "is_cuda")
+
+
+def _check_sc16(items, ndim):
+    """IN_SC16 items are int16 (I, Q) pairs: an int16 array or tensor of `ndim` dimensions whose last one is 2 (push: [n, 2],
+    push_batch: [captures, items, 2]).  A file written by rx_samples_to_file is np.fromfile(path, np.int16).reshape(-1, 2).
+    Returns the items (a numpy array as an ndarray); raises TypeError / ValueError for anything else."""
+    if _is_tensor(items):
+        dt = str(items.dtype).replace("torch.", "")
+    else:
+        if not isinstance(items, np.ndarray):
+            raise TypeError("sc16 items are an int16 numpy array or tensor of shape [..., 2], got %s" % type(items).__name__)
+        dt = str(items.dtype)
+    if dt != "int16":
+        raise TypeError("sc16 items are int16 (I, Q) pairs, got %s" % dt)
+    shape = tuple(items.shape)
+    if len(shape) != ndim or shape[-1] != 2:
+        want = "[n, 2]" if ndim == 2 else "[captures, items, 2]"
+        raise ValueError("sc16 items have shape %s (I, Q last), got %s" % (want, list(shape)))
+    return items
 
 
 def _ptr_and_mem(items, input_kind=None):
     """(address, item count, mem kind, keepalive) of a numpy array or a torch tensor.  A tensor must already hold items of the
-    stream's input kind (one element = one item): the kernels read t.numel() items of that size behind the pointer."""
+    stream's input kind (one element = one item): the kernels read t.numel() items of that size behind the pointer.  IN_SC16:
+    one item is a row of two int16 elements, so the count is the number of rows."""
+    per_item = 2 if input_kind == IN_SC16 else 1
     if hasattr(items, "data_ptr") and hasattr(items, "is_cuda"):  # torch tensor
         if input_kind is not None:
             want = _torch_dtype_name(input_kind)
@@ -140,12 +166,13 @@ def _ptr_and_mem(items, input_kind=None):
             # the library reads device items on its own CUDA stream: whatever produced them on torch's stream must be done
             import torch
             torch.cuda.current_stream(t.device).synchronize()
-        return t.data_ptr(), t.numel(), (MEM_DEVICE if t.is_cuda else MEM_HOST), t
+        return t.data_ptr(), t.numel() // per_item, (MEM_DEVICE if t.is_cuda else MEM_HOST), t
     a = np.ascontiguousarray(items)
-    return a.ctypes.data, a.size, MEM_HOST, a
+    return a.ctypes.data, a.size // per_item, MEM_HOST, a
 
 
-_KIND_DTYPES = {IN_ENVELOPE_F32: np.float32, IN_REAL_F32: np.float32, IN_IQ_F32: np.complex64, IN_PCM_S16: np.int16}
+_KIND_DTYPES = {IN_ENVELOPE_F32: np.float32, IN_REAL_F32: np.float32, IN_IQ_F32: np.complex64, IN_PCM_S16: np.int16,
+                IN_SC16: np.int16}
 
 
 class Stream(object):
@@ -182,8 +209,10 @@ class Stream(object):
         self.params.lo_val, self.params.hi_val = float(lo_val), float(hi_val)
 
     def push(self, items):
-        """-> (consumed, called_back): transition_sink.work semantics (transition_sink.py:37-125)."""
-        if not (hasattr(items, "data_ptr") and hasattr(items, "is_cuda")):
+        """-> (consumed, called_back): transition_sink.work semantics (transition_sink.py:37-125).  IN_SC16: items is [n, 2]."""
+        if self.input_kind == IN_SC16:
+            _check_sc16(items, 2)
+        elif not _is_tensor(items):
             items = np.ascontiguousarray(items, dtype=_KIND_DTYPES[self.input_kind])
         addr, n, mem, keep = _ptr_and_mem(items, self.input_kind)
         cb = C.c_int(0)
@@ -197,8 +226,22 @@ class Stream(object):
         """A batch of independent captures in one pass: items is a 2-D array / tensor [captures, items per capture] of the
         stream's input kind (every row its own transition_sink + decoders in the reference, decoder.py:16-33); lo_vals /
         hi_vals: per-capture thresholds.  Returns the pitch of the position space the results use (capture = pos // pitch,
-        index inside the capture = pos % pitch).  Raises BatchNeedsSequential when a capture must take the sequential path."""
-        if hasattr(items, "data_ptr") and hasattr(items, "is_cuda"):
+        index inside the capture = pos % pitch).  Raises BatchNeedsSequential when a capture must take the sequential path.
+        IN_SC16: items is 3-D, [captures, items per capture, 2] int16."""
+        if self.input_kind == IN_SC16:
+            _check_sc16(items, 3)
+            if _is_tensor(items):
+                keep = items if (items.stride(2) == 1 and items.stride(1) == 2 and items.stride(0) % 2 == 0) else items.contiguous()
+                if keep.is_cuda:
+                    import torch
+                    torch.cuda.current_stream(keep.device).synchronize()  # the library reads the items on its own CUDA stream
+                ncap, n, stride = int(keep.shape[0]), int(keep.shape[1]), int(keep.stride(0)) // 2
+                addr, mem = keep.data_ptr(), (MEM_DEVICE if keep.is_cuda else MEM_HOST)
+            else:
+                keep = np.ascontiguousarray(items)
+                ncap, n, stride = int(keep.shape[0]), int(keep.shape[1]), int(keep.shape[1])
+                addr, mem = keep.ctypes.data, MEM_HOST
+        elif _is_tensor(items):
             if items.dim() != 2:
                 raise ValueError("push_batch takes a 2-D tensor")
             want = _torch_dtype_name(self.input_kind)
@@ -242,7 +285,10 @@ class Stream(object):
 
     def push_all(self, items, chunk=None):
         """Feed everything, re-offering what a call did not consume (the GNU Radio scheduler's job)."""
-        n = items.numel() if hasattr(items, "numel") else len(items)
+        if self.input_kind == IN_SC16:
+            n = len(_check_sc16(items, 2))  # rows of (I, Q)
+        else:
+            n = items.numel() if hasattr(items, "numel") else len(items)
         off = 0
         step = chunk or n
         while off < n:

@@ -44,7 +44,7 @@ struct __align__(8) FrameRec {
 };
 
 // ---- slicer parameters -------------------------------------------------------------------
-enum InputKind { IN_ENVELOPE_F32 = 0, IN_REAL_F32 = 1, IN_IQ_F32 = 2, IN_PCM_S16 = 3 };
+enum InputKind { IN_ENVELOPE_F32 = 0, IN_REAL_F32 = 1, IN_IQ_F32 = 2, IN_PCM_S16 = 3, IN_SC16 = 4 };
 
 struct SlicerParams {
     double lo, hi;   // lo_val, hi_val (transition_sink.py:32-33)
@@ -56,7 +56,7 @@ struct SlicerParams {
     int cls_ss0_xn;  // class when ss == 0 and bit != 0 (ratio = hi + 0.1) transition_sink.py:62-63
     int span_limit;  // max (emax - emin) of admitted exponents for which double sums are exact
     int input_kind;
-    float pcm_scale; // divisor applied to int16 PCM (blocks.wavfile_source), IN_PCM_S16 only
+    float pcm_scale; // divisor applied to int16 samples: PCM (blocks.wavfile_source) and sc16 I / Q
 };
 
 // Slicer state that crosses tiles, segments, slabs and pushes.  The ring itself (L floats) is

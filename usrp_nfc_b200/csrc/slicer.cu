@@ -70,8 +70,24 @@ __device__ __forceinline__ int cta_sync_or(int pred) {
 // ---------------------------------------------------------------- sample loading / envelope
 __device__ __forceinline__ float env_real(float s) { return __fmul_rn(s, s); }  // float_to_complex + mag^2, im = 0
 __device__ __forceinline__ float env_iq(float re, float im) { return __fadd_rn(__fmul_rn(re, re), __fmul_rn(im, im)); }
+// complex int16 (UHD's sc16): the IQ envelope of (I / scale, Q / scale), divided as int16 PCM is
+__device__ __forceinline__ float env_sc16(short2 s, float scale) {
+    return env_iq(__fdiv_rn((float)s.x, scale), __fdiv_rn((float)s.y, scale));
+}
+// four sc16 items read as one 16-byte vector (any 16-byte type): item j is word j, I in its low half
+__device__ __forceinline__ float env_sc16_word(unsigned u, float scale) {
+    return env_sc16(make_short2((short)(u & 0xffffu), (short)(u >> 16)), scale);
+}
+__device__ __forceinline__ float4 env_sc16x4(float4 v, float scale) {
+    return make_float4(env_sc16_word(__float_as_uint(v.x), scale), env_sc16_word(__float_as_uint(v.y), scale),
+                       env_sc16_word(__float_as_uint(v.z), scale), env_sc16_word(__float_as_uint(v.w), scale));
+}
 
+// SC16 = false: code for a kernel that is never launched on sc16 input (the streaming kernel of another kind), which then
+// carries no sc16 branch at all
+template <bool SC16 = true>
 __device__ __forceinline__ float load_one(const void *in, int64_t idx, const SlicerParams &p) {
+    if (SC16 && p.input_kind == IN_SC16) return env_sc16(__ldg(reinterpret_cast<const short2 *>(in) + idx), p.pcm_scale);
     switch (p.input_kind) {
         case IN_ENVELOPE_F32: return __ldg(reinterpret_cast<const float *>(in) + idx);
         case IN_REAL_F32: return env_real(__ldg(reinterpret_cast<const float *>(in) + idx));
@@ -79,7 +95,7 @@ __device__ __forceinline__ float load_one(const void *in, int64_t idx, const Sli
             float2 c = __ldg(reinterpret_cast<const float2 *>(in) + idx);
             return env_iq(c.x, c.y);
         }
-        default: {
+        default: {  // IN_PCM_S16
             float s = __fdiv_rn((float)__ldg(reinterpret_cast<const short *>(in) + idx), p.pcm_scale);
             return env_real(s);
         }
@@ -95,7 +111,7 @@ __device__ __forceinline__ float4 ldg_stream4(const float4 *ptr) {
     return r;
 }
 
-template <int K>
+template <int K, bool SC16 = true>
 __device__ __forceinline__ void load_samples(const SegWork &w, const SlicerParams &p, int64_t p0, float (&x)[K]) {
     const int64_t i0 = p0 - w.in_pos0;
     if (K == 4 && p0 >= w.in_begin && p0 + 4 <= w.in_end) {
@@ -122,11 +138,17 @@ __device__ __forceinline__ void load_samples(const SegWork &w, const SlicerParam
             x[3] = env_real(__fdiv_rn((float)s.w, p.pcm_scale));
             return;
         }
+        if (SC16 && p.input_kind == IN_SC16) {
+            const float4 v = env_sc16x4(ldg_stream4(reinterpret_cast<const float4 *>(reinterpret_cast<const short2 *>(w.in) + i0)),
+                                        p.pcm_scale);
+            x[0] = v.x; x[1] = v.y; x[2] = v.z; x[3] = v.w;
+            return;
+        }
     }
 #pragma unroll
     for (int j = 0; j < K; j++) {
         int64_t q = p0 + j;
-        x[j] = (q >= w.in_begin && q < w.in_end) ? load_one(w.in, q - w.in_pos0, p) : 0.0f;
+        x[j] = (q >= w.in_begin && q < w.in_end) ? load_one<SC16>(w.in, q - w.in_pos0, p) : 0.0f;
     }
 }
 
@@ -248,7 +270,7 @@ __device__ __forceinline__ void exp_track(float x, int &emin, int &emax) {
 // ---------------------------------------------------------------- exact tile (fix-point over prefix sums)
 // One tile of NT*K samples starting at stream index P0, classes decided with every sample's own exact ss.
 // Always correct (inside the exactly-summable regime); several block barriers per tile.
-template <int NT, int K, bool BM = false>
+template <int NT, int K, bool BM = false, bool SC16 = true>
 __device__ __noinline__ void exact_tile(const SegWork *wp, const SlicerParams *pp, float *ring, BlockShared<NT> *shp,
                                         const int64_t P0, const int slot0, SegCarry *cs) {
     constexpr int NW = NT / 32;
@@ -266,7 +288,7 @@ __device__ __noinline__ void exact_tile(const SegWork *wp, const SlicerParams *p
 
     float x[K], prev[K];
     bool act[K];
-    load_samples<K>(w, p, p0, x);
+    load_samples<K, SC16>(w, p, p0, x);
 #pragma unroll
     for (int j = 0; j < K; j++) act[j] = (p0 + j >= w.warm_begin) && (p0 + j < w.end);
 
@@ -864,10 +886,11 @@ template <int KIND>
 static FastVariant fast_variant(int L) {
     static const int pipe = env_int("NFC_SLICER_PIPE", 1), stages = env_int("NFC_SLICER_STAGES", 3);
     const size_t ring = ((size_t)L * 4 + 15) / 16 * 16;
-    const size_t item = KIND == IN_IQ_F32 ? 8 : (KIND == IN_PCM_S16 ? 2 : 4);
+    const size_t item = KIND == IN_IQ_F32 ? 8 : (KIND == IN_PCM_S16 ? 2 : 4);  // IN_SC16: 4, as the float kinds
     const size_t T = L >= FAST_BIG_MIN_L ? 4096 : 512;
     const size_t one = KIND == IN_IQ_F32 ? 0 : T * item;  // staging buffer of the synchronous loop (IQ tiles are not staged)
-    const size_t stg = KIND == IN_PCM_S16 ? T * 6 : T * 4;  // a stage of the pipelined mode (PipeStage): samples, undo log
+    // a stage of the pipelined mode (PipeStage): samples, undo log (4-byte items, sc16 included: the log overlays the samples)
+    const size_t stg = KIND == IN_PCM_S16 ? T * 6 : T * 4;
     const size_t half = smem_optin_limit() / 2;               // two CTAs per SM
     FastVariant v;
     v.tile = (int)T;
@@ -920,6 +943,7 @@ static FastVariant fast_variant_of(int L, int kind) {
         case IN_ENVELOPE_F32: return fast_variant<IN_ENVELOPE_F32>(L);
         case IN_REAL_F32: return fast_variant<IN_REAL_F32>(L);
         case IN_IQ_F32: return fast_variant<IN_IQ_F32>(L);
+        case IN_SC16: return fast_variant<IN_SC16>(L);
         default: return fast_variant<IN_PCM_S16>(L);
     }
 }

@@ -338,7 +338,7 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
     constexpr int T = NW * WS;            // samples per tile
     constexpr int SUB = NT * 4;           // exact_tile row
     constexpr int XR = T / SUB;           // exact_tile rows per tile
-    constexpr int ITEM = KIND == IN_IQ_F32 ? 8 : (KIND == IN_PCM_S16 ? 2 : 4);
+    constexpr int ITEM = KIND == IN_IQ_F32 ? 8 : (KIND == IN_PCM_S16 ? 2 : 4);  // IN_SC16: 4 (I, Q int16)
     constexpr int tile_bytes = T * ITEM;
     static_assert(NC <= 32 && NC >= 4, "one lane per chunk record");
     static_assert(T % SUB == 0, "tile is a whole number of exact rows");
@@ -422,7 +422,7 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
             double part = 0.0, cnt = 0.0;
             for (int i = threadIdx.x; i < L; i += NT) {
                 const int64_t q = w.warm_begin - L + i;
-                float v = load_one(w.in, q - w.in_pos0, p);
+                float v = load_one<KIND == IN_SC16>(w.in, q - w.in_pos0, p);
                 ring[(int)(q % L)] = v;
                 part += (double)v;
             }
@@ -540,6 +540,7 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
                                env_real(__fdiv_rn((float)sv.z, pcm_scale)), env_real(__fdiv_rn((float)sv.w, pcm_scale)));
         }
         float4 v = *reinterpret_cast<const float4 *>(xbuf + r * (NT * 16));
+        if (KIND == IN_SC16) return env_sc16x4(v, p.pcm_scale);  // the 16 staged bytes are four short2
         if (KIND == IN_REAL_F32) { v.x = env_real(v.x); v.y = env_real(v.y); v.z = env_real(v.z); v.w = env_real(v.w); }
         return v;
     };
@@ -562,7 +563,11 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
                 const float4 a = ldg_stream4(q), b = ldg_stream4(q + 1);
                 xin[r] = make_float4(env_iq(a.x, a.y), env_iq(a.z, a.w), env_iq(b.x, b.y), env_iq(b.z, b.w));
             }
-        } else {
+        } else if (KIND == IN_SC16) {
+            const float pcm_scale = p.pcm_scale;
+#pragma unroll
+            for (int r = 0; r < R; r++) xin[r] = env_sc16x4(ldg_stream4(reinterpret_cast<const float4 *>(src + r * FAST_CH * 4)), pcm_scale);
+        } else {  // IN_PCM_S16
             const float pcm_scale = p.pcm_scale;
 #pragma unroll
             for (int r = 0; r < R; r++) {
@@ -1173,7 +1178,7 @@ __global__ void __launch_bounds__(NT + (PIPE ? 64 : 0), MINB) slicer_fast_kernel
                 if (Pr >= w.end || Pr + SUB <= w.warm_begin) continue;  // block-uniform
                 int s0 = slot_x + r * SUB;
                 while (s0 >= L) s0 -= L;
-                exact_tile<NT, 4, true>(&w_s, &p_s, ring, &sh, Pr, s0, &c_s);
+                exact_tile<NT, 4, true, KIND == IN_SC16>(&w_s, &p_s, ring, &sh, Pr, s0, &c_s);
             }
             if (warp == 0) {
                 const double ss1 = c_s.ss0;

@@ -237,6 +237,8 @@ __device__ __noinline__ int pipe_worker(PipeShared<NW, R, S> &ps, float *ring, c
             if (KIND == IN_PCM_S16) {
                 x4 = make_float4(env_real(__fdiv_rn(x4.x, pcm_scale)), env_real(__fdiv_rn(x4.y, pcm_scale)),
                                  env_real(__fdiv_rn(x4.z, pcm_scale)), env_real(__fdiv_rn(x4.w, pcm_scale)));
+            } else if (KIND == IN_SC16) {
+                x4 = env_sc16x4(x4, pcm_scale);  // loaded as 16 raw bytes: four short2
             } else if (KIND == IN_REAL_F32) {
                 x4.x = env_real(x4.x); x4.y = env_real(x4.y); x4.z = env_real(x4.z); x4.w = env_real(x4.w);
             }

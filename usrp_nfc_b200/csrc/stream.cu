@@ -110,6 +110,7 @@ static size_t item_bytes(int kind) {
     switch (kind) {
         case IN_IQ_F32: return 8;
         case IN_PCM_S16: return 2;
+        case IN_SC16: return 4;  // I, Q: two int16
         default: return 4;
     }
 }
@@ -539,6 +540,13 @@ static float host_env(const void *items, int64_t i, int kind, float pcm_scale) {
         }
         case IN_IQ_F32: {
             volatile float re = ((const float *)items)[2 * i], im = ((const float *)items)[2 * i + 1];
+            volatile float a = re * re, b = im * im;
+            volatile float r = a + b;
+            return r;
+        }
+        case IN_SC16: {
+            const int16_t *iq = (const int16_t *)items + 2 * i;
+            volatile float re = (float)iq[0] / pcm_scale, im = (float)iq[1] / pcm_scale;
             volatile float a = re * re, b = im * im;
             volatile float r = a + b;
             return r;
@@ -1771,6 +1779,10 @@ void nfc_default_params(nfc_params *p) {
 int nfc_stream_create(const nfc_params *p, nfc_stream **out) {
     if (!p || !out) {
         nfc::set_error("null argument");
+        return -1;
+    }
+    if (p->input_kind < NFC_IN_ENVELOPE_F32 || p->input_kind > NFC_IN_SC16) {
+        nfc::set_error("unknown input_kind %d (NFC_IN_ENVELOPE_F32 .. NFC_IN_SC16: 0 .. 4)", (int)p->input_kind);
         return -1;
     }
     int ndev = 0;

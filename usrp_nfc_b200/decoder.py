@@ -18,7 +18,8 @@ from .grcompat import HAVE_GNURADIO, blocks, gr
 
 class frame_sink(gr.sync_block):
     """The GPU end of the flowgraph: consumes items, forwards frames.  in_sig is float32 for the WAV
-    path (raw samples, squared on the device) and complex64 for UHD."""
+    path (raw samples, squared on the device), complex64 for UHD, int16 for 16-bit PCM and (int16, 2) for complex int16
+    (UHD's sc16: one item is an I, Q pair; work() takes [n, 2] views)."""
 
     def __init__(self, samp_rate, on_frame, reader=True, tag=True, hi_val=1.1, lo_val=0.1, av_window=2000, max_len=50,
                  input_kind=_cabi.IN_REAL_F32, device=0, on_frame_bytes=None, coalesce=0):
@@ -26,7 +27,8 @@ class frame_sink(gr.sync_block):
         launches whatever its size.  With coalesce > 0 the items of successive calls are collected (every call still consumes
         all it is offered) and go to the device once at least that many are there: the same frames in the same order, at
         most `coalesce` items later.  0: every call is pushed as it comes."""
-        in_type = {_cabi.IN_IQ_F32: numpy.complex64, _cabi.IN_PCM_S16: numpy.int16}.get(input_kind, numpy.float32)
+        in_type = {_cabi.IN_IQ_F32: numpy.complex64, _cabi.IN_PCM_S16: numpy.int16,
+                   _cabi.IN_SC16: (numpy.int16, 2)}.get(input_kind, numpy.float32)
         gr.sync_block.__init__(self, name="nfc_frame_sink", in_sig=[in_type], out_sig=None)
         self._on_frame = on_frame
         self._on_frame_bytes = on_frame_bytes
@@ -74,6 +76,24 @@ class frame_sink(gr.sync_block):
         return self._stream
 
 
+def read_wav(path, iq=False):
+    """The samples of a 16-bit PCM WAV file as int16: channel 0 ([n]), or with iq=True a 2-channel file's (I, Q) pairs
+    ([n, 2], channel 0 = I, channel 1 = Q: GNU Radio's two-channel wavfile_sink and most SDR recorders write baseband so)."""
+    w = wave.open(path, "rb")
+    try:
+        if w.getsampwidth() != 2:
+            raise ValueError("only 16-bit PCM WAV files are supported without GNU Radio")
+        nch = w.getnchannels()
+        if iq and nch != 2:
+            raise ValueError("an IQ WAV file has two channels (I, Q), %s has %d" % (path, nch))
+        data = numpy.frombuffer(w.readframes(w.getnframes()), dtype="<i2").astype(numpy.int16)
+    finally:
+        w.close()
+    if iq:
+        return data.reshape(-1, 2).copy()
+    return data[::nch].copy()
+
+
 def _load_fsm(fsm_module):
     if fsm_module is not None:
         return fsm_module
@@ -87,7 +107,10 @@ def _load_fsm(fsm_module):
 
 class decoder(gr.hier_block2):
     def __init__(self, src="uhd", dst=None, repeat=False, reader=True, tag=True, samp_rate=2e6, emulator=None,
-                 fsm=None, on_frame=None, device=0, on_frame_bytes=None, **sink_kwargs):
+                 fsm=None, on_frame=None, device=0, on_frame_bytes=None, iq=False, **sink_kwargs):
+        """iq=True: src is complex int16 baseband (UHD's sc16), an [n, 2] int16 array or a 2-channel 16-bit WAV path
+        (channels I, Q), decoded as NFC_IN_SC16 with the thresholds of src="uhd".  Without it an int16 array or a WAV
+        file's channel 0 is real PCM."""
         gr.hier_block2.__init__(self, "decoder",
                                 gr.io_signature(0, 0, 0),  # Input signature
                                 gr.io_signature(0, 0, 0))  # Output signature
@@ -107,21 +130,30 @@ class decoder(gr.hier_block2):
             raise ImportError("decoder needs the reference's fsm module on sys.path, or fsm=/on_frame=")
 
         self._pcm = None
+        iq = bool(iq) and not (isinstance(src, str) and src == "uhd")
         if isinstance(src, str) and src == "uhd":
             hi_val = 1.1  # decoder.py:23
             kind = _cabi.IN_IQ_F32
+        elif iq:
+            hi_val = 1.1  # baseband from the USRP, as src="uhd" (decoder.py:23)
+            kind = _cabi.IN_SC16
         else:
             hi_val = 1.09  # decoder.py:29: may need to be set to 1.05 depending on antenna setup
             kind = _cabi.IN_REAL_F32
         hi_val = sink_kwargs.pop("hi_val", hi_val)
-        if not HAVE_GNURADIO and isinstance(src, str) and src != "uhd":
+        if iq:
+            if isinstance(src, numpy.ndarray):
+                _cabi._check_sc16(src, 2)
+            elif not isinstance(src, str):
+                raise TypeError("iq=True takes an [n, 2] int16 array or a 2-channel 16-bit WAV path")
+        elif not HAVE_GNURADIO and isinstance(src, str) and src != "uhd":
             kind = _cabi.IN_PCM_S16  # no wavfile_source here: read the PCM ourselves, normalise on the device
-        if isinstance(src, numpy.ndarray):
+        elif isinstance(src, numpy.ndarray):
             kind = {numpy.dtype(numpy.int16): _cabi.IN_PCM_S16,
                     numpy.dtype(numpy.complex64): _cabi.IN_IQ_F32}.get(src.dtype, _cabi.IN_REAL_F32)
         self._trans = frame_sink(samp_rate, self._on_frame, reader=reader, tag=tag, hi_val=hi_val, input_kind=kind,
                                  device=device, on_frame_bytes=on_frame_bytes, **sink_kwargs)
-        if HAVE_GNURADIO and isinstance(src, str):  # pragma: no cover - needs GNU Radio
+        if HAVE_GNURADIO and isinstance(src, str) and not iq:  # pragma: no cover - needs GNU Radio
             if src == "uhd":
                 # the source of usrp_src.py:19-30 itself, complex items: the reference's wrapper squares them on the host
                 # (usrp_src.py:31-33) and has a float output, this sink takes IN_IQ_F32 and computes the envelope on the device
@@ -137,12 +169,7 @@ class decoder(gr.hier_block2):
         elif isinstance(src, numpy.ndarray):
             self._pcm = src
         elif isinstance(src, str) and src != "uhd":
-            w = wave.open(src, "rb")
-            if w.getsampwidth() != 2:
-                raise ValueError("only 16-bit PCM WAV files are supported without GNU Radio")
-            data = numpy.frombuffer(w.readframes(w.getnframes()), dtype="<i2")
-            self._pcm = data[:: w.getnchannels()].copy()
-            w.close()
+            self._pcm = read_wav(src, iq=iq)
         else:
             raise RuntimeError("src='uhd' needs GNU Radio and UHD")
 

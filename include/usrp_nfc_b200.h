@@ -109,11 +109,23 @@ int64_t nfc_stream_push(nfc_stream *s, const void *items, int64_t n, int mem, in
  * in one space: capture = pos / *pitch, item index inside the capture = pos % *pitch (*pitch: items_per_capture rounded
  * up to whole tiles).  Events and symbols at indices below av_window or from items_per_capture on belong to no capture
  * (they flush the decoders between captures) and are to be skipped by the consumer; frames never carry such positions.
- * NFC_OUT_DROPPED_EVENTS is not available in this mode.  Needs av_window in [1024, 52000], a multiple of 4, and 16-byte
- * aligned captures.  Returns n_captures; -1 on error; -3 when some capture has to take the sequential path (negative or widely
+ * NFC_OUT_DROPPED_EVENTS is not available in this mode.  Needs av_window in [1024, 52000], a multiple of 4, 16-byte
+ * aligned captures and items_per_capture > av_window.  Returns n_captures; -1 on error; -3 when some capture has to take the sequential path (negative or widely
  * spread samples): decode the captures one by one with nfc_stream_push then.  The stream takes no further items until reset. */
 int64_t nfc_stream_push_batch(nfc_stream *s, const void *items, int mem, int64_t n_captures, int64_t items_per_capture,
                               int64_t stride_items, const double *lo_vals, const double *hi_vals, int64_t *pitch);
+
+/* A batch of independent captures of any lengths in one pass: capture c is lengths[c] items of the stream's input kind at
+ * items[c] (all in host memory or all in device memory, per mem; device items 16-byte aligned, host items are staged by the
+ * library).  Otherwise as nfc_stream_push_batch (same stream requirements, lo_vals / hi_vals, -1 / -3 returns, no
+ * NFC_OUT_DROPPED_EVENTS).  starts (n_captures + 1 entries, written): capture c owns the positions [starts[c], starts[c + 1])
+ * of the batch's position space, and its item i is at position starts[c] + i.  starts[0] = 0, starts[c + 1] = starts[c] +
+ * lengths[c] rounded up to whole tiles, or + 0 for a capture of at most av_window items (the warm-up consumes it and nothing
+ * is emitted: transition_sink.py:109-125).  The capture of a frame at pos is the last c with starts[c] <= pos.  A capture of
+ * 2^30 positions or more is refused: decode it with nfc_stream_push.  nfc_stream_push_batch is this call with items[c] =
+ * items + c * stride_items and equal lengths (starts[c] = c * pitch). */
+int64_t nfc_stream_push_batch_ragged(nfc_stream *s, const void *const *items, int mem, int64_t n_captures,
+                                     const int64_t *lengths, const double *lo_vals, const double *hi_vals, int64_t *starts);
 
 /* background.append(transitions) (background.py:27-29): the list transition_sink hands to its callback, fed directly -- the
  * decoders, PacketProcessors and everything behind them run on the device as for pushed samples; decoder and framer state

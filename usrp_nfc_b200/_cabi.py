@@ -62,6 +62,8 @@ SIGNATURES = {
     "nfc_stream_push": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.POINTER(C.c_int)]),
     "nfc_stream_push_batch": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
                                           C.POINTER(C.c_int64)]),
+    "nfc_stream_push_batch_ragged": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p]),
     "nfc_stream_push_events": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64]),
     "nfc_stream_drain_events": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64]),
     "nfc_stream_drain_symbols": (C.c_int64, [C.c_void_p, C.c_void_p, C.c_int64]),
@@ -273,6 +275,69 @@ class Stream(object):
         if rc < 0:
             raise NfcError("nfc_stream_push_batch: " + last_error())
         return int(pitch.value)
+
+    def push_batch_ragged(self, captures, lo_vals=None, hi_vals=None):
+        """A batch of independent captures of any lengths in one pass (as push_batch otherwise): captures is a list of 1-D
+        numpy arrays or CUDA tensors of the stream's input kind ([n_i, 2] int16 for IN_SC16), all on the host or all on the
+        device.  Returns starts (int64, one more entry than captures): capture c owns the positions [starts[c], starts[c + 1])
+        of the results, its item i is at starts[c] + i; a capture of at most av_window items owns none and yields nothing.
+        Raises BatchNeedsSequential when a capture must take the sequential path."""
+        sc16 = self.input_kind == IN_SC16
+        keep, ptrs, lens, mems = [], [], [], set()
+        devices = set()
+        for x in captures:
+            if sc16:
+                _check_sc16(x, 2)
+            if _is_tensor(x):
+                if not sc16:
+                    if x.dim() != 1:
+                        raise ValueError("push_batch_ragged takes 1-D tensors")
+                    want = _torch_dtype_name(self.input_kind)
+                    if str(x.dtype).replace("torch.", "") != want:
+                        raise TypeError("stream input kind %d takes %s items, got a tensor of %s" % (self.input_kind, want, x.dtype))
+                t = x.contiguous()
+                if t.is_cuda and t.data_ptr() % 16:
+                    t = t.clone()  # the library reads device captures from 16-byte aligned addresses
+                mems.add(MEM_DEVICE if t.is_cuda else MEM_HOST)
+                if t.is_cuda:
+                    devices.add(t.device)
+                keep.append(t)
+                ptrs.append(t.data_ptr())
+                lens.append(int(t.shape[0]))
+            else:
+                a = np.ascontiguousarray(x) if sc16 else np.ascontiguousarray(x, dtype=_KIND_DTYPES[self.input_kind])
+                if not sc16 and a.ndim != 1:
+                    raise ValueError("push_batch_ragged takes 1-D arrays")
+                mems.add(MEM_HOST)
+                keep.append(a)
+                ptrs.append(a.ctypes.data)
+                lens.append(int(a.shape[0]))
+        if len(mems) > 1:
+            raise ValueError("push_batch_ragged: the captures are all in host memory or all on the device, not both")
+        ncap = len(keep)
+        if ncap == 0:
+            raise ValueError("push_batch_ragged: no captures")
+        lo = None if lo_vals is None else np.ascontiguousarray(lo_vals, dtype=np.float64)
+        hi = None if hi_vals is None else np.ascontiguousarray(hi_vals, dtype=np.float64)
+        for v in (lo, hi):
+            if v is not None and v.size != ncap:
+                raise ValueError("one threshold per capture")
+        if devices:
+            import torch
+            for d in devices:
+                torch.cuda.current_stream(d).synchronize()  # the library reads the items on its own CUDA stream
+        items = (C.c_void_p * ncap)(*ptrs)
+        lengths = np.ascontiguousarray(lens, dtype=np.int64)
+        starts = np.zeros(ncap + 1, dtype=np.int64)
+        rc = lib().nfc_stream_push_batch_ragged(self._h, items, mems.pop(), ncap, lengths.ctypes.data,
+                                                None if lo is None else lo.ctypes.data, None if hi is None else hi.ctypes.data,
+                                                starts.ctypes.data)
+        del keep
+        if rc == -3:
+            raise BatchNeedsSequential(last_error())
+        if rc < 0:
+            raise NfcError("nfc_stream_push_batch_ragged: " + last_error())
+        return starts
 
     def push_events(self, events):
         """background.append (background.py:27-29): transition_sink's events (EVENT_DTYPE array: pos, d, v, type) straight

@@ -82,23 +82,33 @@ def decode_batch(captures, samp_rate, params, device=0, workers=8, tuning=None, 
 
 def decode_batch_onepass(captures, samp_rate, params, lo_vals=None, hi_vals=None, device=0, outputs=_cabi.OUT_FRAMES,
                          kind=_cabi.IN_ENVELOPE_F32, stream=None):
-    """A batch of equally long captures in one pass over the device (nfc_stream_push_batch): one launch of the slicer with
-    one segment per capture, extraction / runs / line code over the whole batch, no host work per capture.
+    """A batch of captures in one pass over the device (nfc_stream_push_batch / nfc_stream_push_batch_ragged): one launch
+    of the slicer with one segment per capture, extraction / runs / line code over the whole batch, no host work per
+    capture.
 
-    captures: 2-D array or CUDA tensor [captures, items]; params: the Stream keyword arguments all captures share
-    (av_window, max_len, ...); lo_vals / hi_vals: one threshold per capture (transition_sink's constructor arguments,
-    transition_sink.py:12).  stream: a Stream to reuse (it is reset).  Returns dict(pitch, frames, bits_tag, bits_reader,
-    stream): frame records with positions in the batch's position space (capture = pos // pitch, index inside the
-    capture = pos % pitch), bit_off into bits_tag (type 0) / bits_reader (type 1); views valid until the stream is used
-    again.  Falls back to decode_batch when a capture needs the sequential path (the same results, capture by capture)."""
+    captures: 2-D array or CUDA tensor [captures, items] of equally long captures, or a list of 1-D arrays or CUDA tensors
+    of any lengths (all on the host or all on the device; IN_SC16: [items, 2] int16 each); params: the Stream keyword
+    arguments all captures share (av_window, max_len, ...); lo_vals / hi_vals: one threshold per capture (transition_sink's
+    constructor arguments, transition_sink.py:12).  stream: a Stream to reuse (it is reset).  Returns dict(starts, pitch,
+    frames, bits_tag, bits_reader, stream): frame records with positions in the batch's position space (capture c owns
+    [starts[c], starts[c + 1]), its item i is at starts[c] + i; pitch: the distance between captures of a 2-D batch, None for
+    a list), bit_off into bits_tag (type 0) / bits_reader (type 1); views valid until the stream is used again.  Falls back
+    to decode_batch when a capture needs the sequential path (the same results, capture by capture).
+
+    Every capture is one segment on one CTA: a capture far longer than the rest bounds the batch's time at one CTA's rate."""
     s = stream
     if s is None:
         s = _cabi.Stream(samp_rate, device=device, outputs=outputs, input_kind=kind, **params)
     else:
         s.release_frames()
         s.reset()
+    ragged = isinstance(captures, (list, tuple))
     try:
-        pitch = s.push_batch(captures, lo_vals=lo_vals, hi_vals=hi_vals)
+        if ragged:
+            starts, pitch = s.push_batch_ragged(captures, lo_vals=lo_vals, hi_vals=hi_vals), None
+        else:
+            pitch = s.push_batch(captures, lo_vals=lo_vals, hi_vals=hi_vals)
+            starts = np.arange(len(captures) + 1, dtype=np.int64) * pitch
     except _cabi.BatchNeedsSequential:
         n = len(captures)
         plist = []
@@ -110,9 +120,9 @@ def decode_batch_onepass(captures, samp_rate, params, lo_vals=None, hi_vals=None
                 p["hi_val"] = float(hi_vals[i])
             plist.append(p)
         res = decode_batch([captures[i] for i in range(n)], samp_rate, plist, device=device, outputs=outputs, kind=kind)
-        return dict(pitch=None, per_capture=res, stream=s)
+        return dict(starts=None, pitch=None, per_capture=res, stream=s)
     fr, b0, b1 = s.view_frames()
-    return dict(pitch=pitch, frames=fr, bits_tag=b0, bits_reader=b1, stream=s)
+    return dict(starts=starts, pitch=pitch, frames=fr, bits_tag=b0, bits_reader=b1, stream=s)
 
 
 def split_captures(res, n_captures):
@@ -120,8 +130,12 @@ def split_captures(res, n_captures):
     positions relative to the capture, bit_off into the capture's own bit array."""
     if res.get("per_capture") is not None:
         return res["per_capture"]
-    fr, pitch = res["frames"], res["pitch"]
-    cap = fr["pos"] // pitch
+    fr = res["frames"]
+    starts = res.get("starts")
+    if starts is None:
+        starts = np.arange(n_captures + 1, dtype=np.int64) * res["pitch"]
+    starts = np.asarray(starts, dtype=np.int64)
+    cap = np.searchsorted(starts, fr["pos"], "right") - 1
     out = []
     for c in range(n_captures):
         sel = fr[cap == c].copy()
@@ -132,7 +146,7 @@ def split_captures(res, n_captures):
             bits.append(np.array(src[int(r["bit_off"]): int(r["bit_off"]) + int(r["nbits"])], dtype=np.uint8))
             r["bit_off"] = off
             off += int(r["nbits"])
-        sel["pos"] -= c * pitch
+        sel["pos"] -= starts[c]
         out.append((sel, np.concatenate(bits) if bits else np.zeros(0, np.uint8)))
     return out
 

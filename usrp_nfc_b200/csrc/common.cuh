@@ -151,11 +151,18 @@ struct LineTables {
     int n_dclass_miller, n_dclass_manch;
     int decode_reader, decode_tag;
     // A batch of independent captures decoded as one event stream (every capture its own transition_sink, decoders and
-    // PacketProcessors in the reference: transition_sink.py:12-34, background.py:17-25): capture k of a slab owns the
-    // slab-relative positions [k * batch_pitch, (k + 1) * batch_pitch); only events at offsets [batch_skip, batch_len) of it
-    // are the capture's (before: its warm-up, transition_sink.py:109-125; behind: padding), the others are ignored; the first
-    // event of a capture finds both decoders and both PacketProcessors as new.  batch_pitch == 0: one stream.
-    uint32_t batch_pitch, batch_skip, batch_len;
+    // PacketProcessors in the reference: transition_sink.py:12-34, background.py:17-25).  batch_tab (device memory, valid
+    // while any chain of the batch may still run or be done again): batch_n + 1 start positions, then batch_n lengths;
+    // capture k owns the batch positions [start[k], start[k + 1]).  Only events at offsets [batch_skip, length[k]) of it are
+    // the capture's (before: its warm-up, transition_sink.py:109-125; behind: padding), the others are ignored; the first
+    // event of a capture finds both decoders and both PacketProcessors as new.  A slab begins with capture batch_c0 at batch
+    // position batch_base (event positions are relative to it).  batch_tab == nullptr: one stream.
+    // What the run carry brings into a capture cannot leak into its events: its own range is preceded by its warm-up, batch_skip
+    // = av_window positions of val == 0, and av_window > max_len + 1, so the run crossing the boundary has timed out and
+    // reset cur_state (transition_sink.py:95-99) before the capture's first own sample, whatever the capture before left.
+    const int64_t *batch_tab;
+    int64_t batch_base;
+    uint32_t batch_n, batch_c0, batch_skip;
 };
 
 struct DecCarry {

@@ -95,19 +95,57 @@ struct TabView {
     const TabEntry *tab;            // tables (one shared memory copy: Miller, then Manchester at goff)
     int goff;
     int use_reader, use_tag;
-    uint32_t pitch, skip, len;      // batches of captures (LineTables::batch_*); pitch == 0: one stream
+    // batches of captures (LineTables::batch_*); caps == nullptr: one stream
+    const int64_t *caps;
+    int64_t base;
+    int n_caps, c0;
+    uint32_t skip;
 };
 
-// Batches of captures: which capture an event belongs to, and whether it is one of the capture's own events.
-static const uint32_t NO_CAPTURE = 0xffffffffu;
-__device__ __forceinline__ uint32_t batch_capture(const TabView &tv, uint32_t rel_pos, bool &inside) {
-    const uint32_t cap = rel_pos / tv.pitch, off = rel_pos - cap * tv.pitch;
-    inside = off >= tv.skip && off < tv.len;
-    return cap;
+// Batches of captures: which capture an event belongs to, and whether it is one of the capture's own events.  Events come
+// in position order, so a walk over events keeps a cursor in the capture table: one binary search where the walk begins,
+// then a step to the next capture whenever an event passes its start.
+struct CapCursor {
+    int k;             // capture of the last event walked over (c0 - 1 before the slab's first event)
+    uint32_t lo, hi;   // its own events: slab-relative positions [start + skip, start + length)
+    uint32_t next;     // slab-relative start of capture k + 1
+};
+__device__ __forceinline__ uint32_t cap_rel(const TabView &tv, int64_t p) {  // batch position -> slab-relative (clamped)
+    const int64_t r = p - tv.base;
+    return r < 0 ? 0u : (r > (int64_t)0xffffffffu ? 0xffffffffu : (uint32_t)r);
 }
-// the capture of the event before event i (NO_CAPTURE before the slab's first event: a slab starts with a capture)
-__device__ __forceinline__ uint32_t batch_capture_before(const TabView &tv, const EventRec *__restrict__ ev, int64_t i) {
-    return i > 0 ? ev[i - 1].rel_pos / tv.pitch : NO_CAPTURE;
+__device__ __forceinline__ void cap_load(const TabView &tv, CapCursor &cc, int k) {
+    const int64_t s = tv.caps[k], len = tv.caps[tv.n_caps + 1 + k];
+    cc.k = k;
+    cc.lo = cap_rel(tv, s + tv.skip);
+    cc.hi = cap_rel(tv, s + len);
+    cc.next = cap_rel(tv, tv.caps[k + 1]);
+}
+// the cursor at the capture of event i - 1 (before the slab's first capture when i == 0: a slab starts with a capture)
+__device__ __forceinline__ void cap_seek(const TabView &tv, CapCursor &cc, const EventRec *__restrict__ ev, int64_t i) {
+    if (i <= 0) {
+        cc.k = tv.c0 - 1;
+        cc.lo = cc.hi = cc.next = 0;
+        return;
+    }
+    const int64_t p = tv.base + (int64_t)ev[i - 1].rel_pos;
+    int lo = tv.c0, hi = tv.n_caps - 1;  // the last capture that starts at or before p (empty captures start where the next does)
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (tv.caps[mid] <= p) lo = mid;
+        else hi = mid - 1;
+    }
+    cap_load(tv, cc, lo);
+}
+// moves the cursor to the capture of an event at rel_pos; true when that is another capture than the last event's
+__device__ __forceinline__ bool cap_step(const TabView &tv, CapCursor &cc, uint32_t rel_pos, bool &inside) {
+    bool changed = false;
+    while (rel_pos >= cc.next && cc.k + 1 < tv.n_caps) {
+        cap_load(tv, cc, cc.k + 1);
+        changed = true;
+    }
+    inside = rel_pos >= cc.lo && rel_pos < cc.hi;
+    return changed;
 }
 
 // one symbol into a PacketProcessor (packets.py:67-79); returns 1 when a frame is closed
@@ -148,14 +186,13 @@ __device__ __forceinline__ void step_event(const EventRec &ev, const TabView &tv
 }
 
 // the same for a stream that may be a batch of captures: a capture's first event finds everything as new
-// (background.py:17-25, packets.py:63-65), events outside a capture's own range are ignored
-template <class Sink>
-__device__ __forceinline__ void step_event_batch(const EventRec &ev, const TabView &tv, int &rs, int &gs, Sink &sink, uint32_t &cap_prev) {
-    if (tv.pitch) {
+// (background.py:17-25, packets.py:63-65), events outside a capture's own range are ignored.  The kernels are instantiated
+// for single streams (BATCH = false: no capture lookup in the event loops) and for batches.
+template <bool BATCH, class Sink>
+__device__ __forceinline__ void step_event_batch(const EventRec &ev, const TabView &tv, int &rs, int &gs, Sink &sink, CapCursor &cur) {
+    if (BATCH) {
         bool inside;
-        const uint32_t cap = batch_capture(tv, ev.rel_pos, inside);
-        if (cap != cap_prev) {
-            cap_prev = cap;
+        if (cap_step(tv, cur, ev.rel_pos, inside)) {
             rs = 0;
             gs = 0;
             sink.new_capture();
@@ -168,18 +205,21 @@ __device__ __forceinline__ void step_event_batch(const EventRec &ev, const TabVi
 // eight events at once (one 64-byte line): the loops below are chains of dependent loads otherwise.
 // `base` is a multiple of 8; the event buffer is padded, so reading a little past n_ev is safe.
 __device__ __forceinline__ void load8(const EventRec *__restrict__ ev, int64_t base, EventRec (&e)[8]) {
-    const uint4 *p = reinterpret_cast<const uint4 *>(ev + base);
-    const uint4 q[4] = {__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3)};
+    // In 64-bit lanes, so that the single-stream kernels, which read no positions, still load 16 bytes at a time: with
+    // 32-bit lanes the compiler drops the position words and issues eight 4-byte loads, which made the chains slower.
+    const ulonglong2 *p = reinterpret_cast<const ulonglong2 *>(ev + base);
+    const ulonglong2 q[4] = {__ldg(p), __ldg(p + 1), __ldg(p + 2), __ldg(p + 3)};
 #pragma unroll
     for (int k = 0; k < 4; k++) {
-        const unsigned w[4] = {q[k].x, q[k].y, q[k].z, q[k].w};
+        const unsigned long long w[2] = {q[k].x, q[k].y};
 #pragma unroll
         for (int h = 0; h < 2; h++) {
+            const unsigned hi = (unsigned)(w[h] >> 32);
             EventRec r;
-            r.rel_pos = w[2 * h];
-            r.d = (uint16_t)(w[2 * h + 1] & 0xffffu);
-            r.v = (int8_t)((w[2 * h + 1] >> 16) & 0xffu);
-            r.type = (int8_t)(w[2 * h + 1] >> 24);
+            r.rel_pos = (unsigned)w[h];
+            r.d = (uint16_t)(hi & 0xffffu);
+            r.v = (int8_t)((hi >> 16) & 0xffu);
+            r.type = (int8_t)(hi >> 24);
             e[2 * k + h] = r;
         }
     }
@@ -205,9 +245,10 @@ __device__ __forceinline__ void load_tables(const LineTables &lt, TabEntry *sm, 
     tv.dcm = lt.dclass_miller; tv.dcg = lt.dclass_manch;            \
     tv.tab = s_tab; tv.goff = MAX_DCLASS * 4 * MILLER_STATES;        \
     tv.use_reader = lt.decode_reader; tv.use_tag = lt.decode_tag;   \
-    tv.pitch = lt.batch_pitch; tv.skip = lt.batch_skip; tv.len = lt.batch_len;
+    tv.caps = lt.batch_tab; tv.base = lt.batch_base; tv.n_caps = (int)lt.batch_n; tv.c0 = (int)lt.batch_c0; tv.skip = lt.batch_skip;
 
 // ---- pass A: transfer function of every chunk -------------------------------------------------
+template <bool BATCH>
 __global__ void chunk_map_kernel(const EventRec *__restrict__ ev, EvCount evc, LineTables lt,
                                  ChunkMap *__restrict__ maps, uint32_t cap_chunks) {
     NFC_TABLE_SMEM
@@ -220,14 +261,13 @@ __global__ void chunk_map_kernel(const EventRec *__restrict__ ev, EvCount evc, L
     for (int s = 0; s < GSTATES; s++) g[s] = (uint8_t)s;
     bool r_flat = false, g_flat = false;  // all start states already lead to the same state
     NullSink sink;
-    uint32_t cap_prev = tv.pitch ? batch_capture_before(tv, ev, (int64_t)i0) : 0u;
+    CapCursor cur;
+    if (BATCH) cap_seek(tv, cur, ev, (int64_t)i0);
     for (uint32_t i = i0; i < i1; i++) {
         const EventRec e = ev[i];
-        if (tv.pitch) {
+        if (BATCH) {
             bool inside;
-            const uint32_t cap = batch_capture(tv, e.rel_pos, inside);
-            if (cap != cap_prev) {  // a new capture: every state leads to the initial one
-                cap_prev = cap;
+            if (cap_step(tv, cur, e.rel_pos, inside)) {  // a new capture: every state leads to the initial one
                 r[0] = 0; g[0] = 0;
                 r_flat = g_flat = true;
             }
@@ -305,6 +345,7 @@ struct CountSink {
 // (per direction) and replays only the events between that chunk's end and its own start (none when it is the previous
 // chunk).  start[c] = R state | G state << 8.  Chunks that find nothing within LOOKBACK_LIMIT events raise *unresolved
 // (the host then takes the transfer-function scan below for the slab).
+template <bool BATCH>
 __global__ void chunk_summary_kernel(const EventRec *__restrict__ ev, EvCount evc, LineTables lt,
                                      uint16_t *__restrict__ summary) {
     NFC_TABLE_SMEM
@@ -315,7 +356,8 @@ __global__ void chunk_summary_kernel(const EventRec *__restrict__ ev, EvCount ev
     bool kR = false, kG = false;
     NullSink sink;
     const uint32_t i0 = c * CHUNK, i1 = min(n_ev, i0 + CHUNK);
-    uint32_t cap_prev = tv.pitch ? batch_capture_before(tv, ev, (int64_t)i0) : 0u;
+    CapCursor cur;
+    if (BATCH) cap_seek(tv, cur, ev, (int64_t)i0);
     for (uint32_t i = i0; i < i1; i += 8) {
         EventRec e8[8];
         load8(ev, i, e8);
@@ -324,11 +366,9 @@ __global__ void chunk_summary_kernel(const EventRec *__restrict__ ev, EvCount ev
             if (i + k >= i1) continue;
             const EventRec e = e8[k];
             int dummy = 0;
-            if (tv.pitch) {
+            if (BATCH) {
                 bool inside;
-                const uint32_t cap = batch_capture(tv, e.rel_pos, inside);
-                if (cap != cap_prev) {  // a new capture: both machines are known to be in their initial state
-                    cap_prev = cap;
+                if (cap_step(tv, cur, e.rel_pos, inside)) {  // a new capture: both machines are known to be in their initial state
                     rs = 0; kR = true;
                     gs = 0; kG = true;
                 }
@@ -348,6 +388,7 @@ __global__ void chunk_summary_kernel(const EventRec *__restrict__ ev, EvCount ev
     summary[c] = (uint16_t)((rs & 31) | (kR ? 32 : 0) | ((gs & 15) << 8) | (kG ? 4096 : 0));
 }
 
+template <bool BATCH>
 __global__ void chunk_start_kernel(const EventRec *__restrict__ ev, EvCount evc, LineTables lt,
                                    const DecCarry *__restrict__ carry_in, const uint16_t *__restrict__ summary,
                                    uint16_t *__restrict__ start, uint32_t *__restrict__ flags) {
@@ -377,7 +418,8 @@ __global__ void chunk_start_kernel(const EventRec *__restrict__ ev, EvCount evc,
     // replay from the earliest point a still-unknown machine needs (a disabled direction needs nothing)
     const int64_t fromR = tv.use_reader ? iR + 1 : i0, fromG = tv.use_tag ? iG + 1 : i0;
     const int64_t from = fromR < fromG ? fromR : fromG;
-    uint32_t cap_prev = (tv.pitch && from < i0) ? batch_capture_before(tv, ev, from) : 0u;
+    CapCursor cur;
+    if (BATCH && from < i0) cap_seek(tv, cur, ev, from);
     for (int64_t base = from & ~(int64_t)7; base < i0; base += 8) {
         EventRec e8[8];
         load8(ev, base, e8);
@@ -387,11 +429,9 @@ __global__ void chunk_start_kernel(const EventRec *__restrict__ ev, EvCount evc,
             if (kk < from || kk >= i0) continue;
             const EventRec e = e8[k];
             int dummy_r = 0, dummy_g = 0;
-            if (tv.pitch) {
+            if (BATCH) {
                 bool inside;
-                const uint32_t cap = batch_capture(tv, e.rel_pos, inside);
-                if (cap != cap_prev) {  // a new capture behind the point a machine's state was known at: initial state
-                    cap_prev = cap;
+                if (cap_step(tv, cur, e.rel_pos, inside)) {  // a new capture behind the point a machine's state was known at: initial state
                     if (kk > iR) rs = 0;
                     if (kk > iG) gs = 0;
                 }
@@ -418,6 +458,7 @@ __global__ void chunk_start_from_maps_kernel(const ChunkMap *__restrict__ prefix
     start[c] = (uint16_t)(prefix[c].r[rs0] | (prefix[c].g[gs0] << 8));
 }
 
+template <bool BATCH>
 __global__ void chunk_count_kernel(const EventRec *__restrict__ ev, EvCount evc, LineTables lt,
                                    const uint16_t *__restrict__ start, ChunkCnt *__restrict__ cnts, uint32_t cap_chunks) {
     NFC_TABLE_SMEM
@@ -432,13 +473,14 @@ __global__ void chunk_count_kernel(const EventRec *__restrict__ ev, EvCount evc,
     }
     int rs = start[c] & 31, gs = (start[c] >> 8) & 15;
     const uint32_t i0 = c * CHUNK, i1 = min(n_ev, i0 + CHUNK);
-    uint32_t cap_prev = tv.pitch ? batch_capture_before(tv, ev, (int64_t)i0) : 0u;
+    CapCursor cur;
+    if (BATCH) cap_seek(tv, cur, ev, (int64_t)i0);
     for (uint32_t i = i0; i < i1; i += 8) {
         EventRec e[8];
         load8(ev, i, e);
 #pragma unroll
         for (int k = 0; k < 8; k++)
-            if (i + k < i1) step_event_batch(e[k], tv, rs, gs, sink, cap_prev);
+            if (i + k < i1) step_event_batch<BATCH>(e[k], tv, rs, gs, sink, cur);
     }
     cnts[c] = sink.c;
 }
@@ -507,6 +549,7 @@ struct LineOut {
     uint32_t *n_frames;                 // records written (the scan's total may count one more per type: ChunkCnt)
 };
 
+template <bool BATCH>
 __global__ void chunk_write_kernel(const EventRec *__restrict__ ev, EvCount evc, LineTables lt,
                                    const uint16_t *__restrict__ start,
                                    const ChunkCnt *__restrict__ cnt_prefix, LineOut out, const DecCarry *__restrict__ carry_in,
@@ -532,13 +575,14 @@ __global__ void chunk_write_kernel(const EventRec *__restrict__ ev, EvCount evc,
     sink.pend0 = (pc.has0 & 1) ? pc.tail0 : out.pending_in[0] + pc.tail0;
     sink.pend1 = (pc.has1 & 1) ? pc.tail1 : out.pending_in[1] + pc.tail1;
     const uint32_t i0 = c * CHUNK, i1 = min(n_ev, i0 + CHUNK);
-    uint32_t cap_prev = tv.pitch ? batch_capture_before(tv, ev, (int64_t)i0) : 0u;
+    CapCursor cur;
+    if (BATCH) cap_seek(tv, cur, ev, (int64_t)i0);
     for (uint32_t i = i0; i < i1; i += 8) {
         EventRec e[8];
         load8(ev, i, e);
 #pragma unroll
         for (int k = 0; k < 8; k++)
-            if (i + k < i1) step_event_batch(e[k], tv, rs, gs, sink, cap_prev);
+            if (i + k < i1) step_event_batch<BATCH>(e[k], tv, rs, gs, sink, cur);
     }
     if (c == n_chunks - 1) {
         DecCarry co;
@@ -568,9 +612,9 @@ int launch_linecode_start(const EventRec *d_ev, const uint32_t *d_M, uint32_t ca
                           uint16_t *d_summary, uint16_t *d_start, uint32_t *d_flags, cudaStream_t stream) {
     const uint32_t nc = std::max(1u, linecode_chunks(cap_ev));
     const EvCount evc{d_M, cap_ev};
-    chunk_summary_kernel<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_summary);
+    (lt.batch_tab ? chunk_summary_kernel<true> : chunk_summary_kernel<false>)<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_summary);
     NFC_CUDA_CHECK(cudaGetLastError());
-    chunk_start_kernel<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_carry_in, d_summary, d_start, d_flags);
+    (lt.batch_tab ? chunk_start_kernel<true> : chunk_start_kernel<false>)<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_carry_in, d_summary, d_start, d_flags);
     NFC_CUDA_CHECK(cudaGetLastError());
     return 0;
 }
@@ -583,7 +627,7 @@ int launch_linecode_start_scan(const EventRec *d_ev, const uint32_t *d_M, uint32
     ChunkMap *maps = (ChunkMap *)d_maps, *prefix = (ChunkMap *)d_prefix;
     const unsigned nb = (nc + 127) / 128;
     const EvCount evc{d_M, cap_ev};
-    chunk_map_kernel<<<nb, 128, 0, stream>>>(d_ev, evc, lt, maps, nc);
+    (lt.batch_tab ? chunk_map_kernel<true> : chunk_map_kernel<false>)<<<nb, 128, 0, stream>>>(d_ev, evc, lt, maps, nc);
     NFC_CUDA_CHECK(cudaGetLastError());
     ChunkMap ident;
     for (int s = 0; s < RSTATES; s++) ident.r[s] = (uint8_t)s;
@@ -601,7 +645,7 @@ int launch_linecode_count(const EventRec *d_ev, const uint32_t *d_M, uint32_t ca
     const uint32_t nc = std::max(1u, linecode_chunks(cap_ev));
     ChunkCnt *cnts = (ChunkCnt *)d_cnts, *cprefix = (ChunkCnt *)d_cnt_prefix;
     const EvCount evc{d_M, cap_ev};
-    chunk_count_kernel<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_start, cnts, nc);
+    (lt.batch_tab ? chunk_count_kernel<true> : chunk_count_kernel<false>)<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_start, cnts, nc);
     NFC_CUDA_CHECK(cudaGetLastError());
     ChunkCnt zero = {0, 0, 0, 0, 0, 0, 0, 0};
     return device_exclusive_scan<ChunkCnt, CombineCnt>(cnts, cprefix, nc, zero, CombineCnt(), (ChunkCnt *)d_scratch,
@@ -624,7 +668,7 @@ int launch_linecode_write(const EventRec *d_ev, const uint32_t *d_M, uint32_t ca
     out.n_empty = d_n_empty;
     out.n_frames = d_n_frames;
     const EvCount evc{d_M, cap_ev};
-    chunk_write_kernel<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_start, (const ChunkCnt *)d_cnt_prefix, out,
+    (lt.batch_tab ? chunk_write_kernel<true> : chunk_write_kernel<false>)<<<(nc + 127) / 128, 128, 0, stream>>>(d_ev, evc, lt, d_start, (const ChunkCnt *)d_cnt_prefix, out,
                                                              d_carry_in, d_carry_out, d_pending_out);
     NFC_CUDA_CHECK(cudaGetLastError());
     return 0;

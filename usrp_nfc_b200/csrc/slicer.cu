@@ -1056,19 +1056,18 @@ int slicer_resident_ctas(int L, int kind) {
 
 // ---------------------------------------------------------------- batches of independent captures
 // The reference gives every capture its own transition_sink (transition_sink.py:12-34): the first av_window items fill the
-// ring unconditionally, _sum is their left-to-right double sum (transition_sink.py:109-125).  One block per capture writes
-// that state as a state block; the ring is laid out by stream position of the batch (capture c starts at c * pitch).
-__global__ void __launch_bounds__(256) batch_warm_kernel(const char *__restrict__ items, int64_t stride_bytes, int64_t pitch,
-                                                         const SlicerParams *__restrict__ params, char *__restrict__ states,
-                                                         size_t state_bytes) {
+// ring unconditionally, _sum is their left-to-right double sum (transition_sink.py:109-125).  One block per segment of the
+// batch (one segment per capture) writes that state into the segment's state_in block; the capture's items are at w.in and
+// its first item has batch position w.in_pos0, by which the ring is laid out.
+__global__ void __launch_bounds__(256) batch_warm_kernel(const SegWork *__restrict__ works, const SlicerParams *__restrict__ params) {
     extern __shared__ float warm_s[];
-    const int64_t c = blockIdx.x;
-    const SlicerParams p = params[c];
+    const SegWork &w = works[blockIdx.x];
+    const SlicerParams p = params[w.param_idx];
     const int L = p.L;
-    SlicerHdr *h = reinterpret_cast<SlicerHdr *>(states + (size_t)c * state_bytes);
+    SlicerHdr *h = const_cast<SlicerHdr *>(w.state_in);
     float *ring = state_ring(h);
-    const int64_t B = c * pitch;
-    const void *in = items + c * stride_bytes;
+    const int64_t B = w.in_pos0;
+    const void *in = w.in;
     for (int i = threadIdx.x; i < L; i += blockDim.x) {
         const float v = load_one(in, i, p);
         warm_s[i] = v;
@@ -1097,12 +1096,11 @@ __global__ void bitmap_fill_kernel(uint4 *__restrict__ bm, size_t n_chunks) {
     bm[2 * i + 1] = make_uint4(0u, 0u, 0u, 0u);
 }
 
-int launch_batch_warm(const void *d_items, int64_t stride_bytes, int64_t pitch, int n_cap, int L, const SlicerParams *d_params,
-                      void *d_states, size_t state_bytes, cudaStream_t stream) {
-    if (n_cap <= 0) return 0;
+int launch_batch_warm(const SegWork *d_works, int n_works, int L, const SlicerParams *d_params, cudaStream_t stream) {
+    if (n_works <= 0) return 0;
     const size_t smem = (size_t)L * 4;
     if (raise_dynamic_smem((const void *)batch_warm_kernel, smem)) return -1;
-    batch_warm_kernel<<<n_cap, 256, smem, stream>>>((const char *)d_items, stride_bytes, pitch, d_params, (char *)d_states, state_bytes);
+    batch_warm_kernel<<<n_works, 256, smem, stream>>>(d_works, d_params);
     NFC_CUDA_CHECK(cudaGetLastError());
     return 0;
 }

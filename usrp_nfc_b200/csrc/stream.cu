@@ -68,8 +68,7 @@ int launch_linecode_write(const EventRec *d_ev, const uint32_t *d_M, uint32_t ca
 int slicer_tile(int L, int kind);
 int slicer_resident_ctas(int L, int kind);
 int slicer_tile_stats(unsigned long long *out4, bool reset);
-int launch_batch_warm(const void *d_items, int64_t stride_bytes, int64_t pitch, int n_cap, int L, const SlicerParams *d_params,
-                      void *d_states, size_t state_bytes, cudaStream_t stream);
+int launch_batch_warm(const SegWork *d_works, int n_works, int L, const SlicerParams *d_params, cudaStream_t stream);
 int launch_bitmap_fill(uint32_t *d_bm, size_t n_chunks, cudaStream_t stream);
 int synth_render(void *dev_out, int64_t n, int64_t first_index, const int8_t *codes, const int64_t *lens, int64_t n_runs,
                  float carrier, float pause, float tag_high, float noise, float fade, double fade_period, uint64_t seed,
@@ -345,9 +344,14 @@ struct Stream {
     int64_t push(const void *items, int64_t n, int mem, int *called_back);
     int64_t push_batch(const void *items, int mem, int64_t n_cap, int64_t cap_len, int64_t stride_items, const double *lo_vals,
                        const double *hi_vals, int64_t *pitch_out);
-    // layout of the class bitmap a batch was filled for (positions no segment writes hold val == 0 and stay so)
-    int64_t batch_fill_pitch = 0, batch_fill_caps = 0, batch_fill_len = 0;
-    DevBuf batch_states, batch_stage;
+    int64_t push_batch_ragged(const void *const *items, int mem, int64_t n_cap, const int64_t *lengths, const double *lo_vals,
+                              const double *hi_vals, int64_t *starts_out);
+    // the segment ranges [start + L, start + length) of the batch the class bitmap was last filled for: positions no segment
+    // of that batch wrote hold val == 0.  A batch whose segments are the same ranges, or a prefix of them, finds the rest of
+    // its positions at val == 0 too; any other layout, and a single stream's slicer, write elsewhere (empty: fill again).
+    std::vector<int64_t> batch_fill;
+    DevBuf batch_states, batch_stage, batch_tab;
+    std::vector<int64_t> batch_starts;  // host copy of the capture table's starts (a slab's first capture: post_chain)
     int finish_warmup();
     int process_slab(const void *d_in, int64_t in_pos0, int64_t in_begin, int64_t in_end, int64_t a, int64_t b, int64_t slicer_end);
     // the streaming kernel writes the class bitmap; the first-generation kernel (windows below 1024 samples or not a
@@ -468,9 +472,9 @@ int Stream::init(const nfc_params *p) {
     lt.n_dclass_manch = ht.n_dclass_manch;
     lt.decode_reader = p->decode_reader;
     lt.decode_tag = p->decode_tag;
-    lt.batch_pitch = 0;
-    lt.batch_skip = 0;
-    lt.batch_len = 0;
+    lt.batch_tab = nullptr;
+    lt.batch_base = 0;
+    lt.batch_n = lt.batch_c0 = lt.batch_skip = 0;
 
     warm.reserve((size_t)sp.L);
     if (state.ensure(state_block_bytes(sp.L))) return -1;
@@ -481,7 +485,7 @@ int Stream::init(const nfc_params *p) {
 }
 
 void Stream::destroy() {
-    DevBuf *all[] = {&batch_states, &batch_stage, &params_d, &tab_d, &staging, &works_d, &states_d, &trans_seg, &trans_dense[0], &trans_dense[1], &seg_counts,
+    DevBuf *all[] = {&batch_states, &batch_stage, &batch_tab, &params_d, &tab_d, &staging, &works_d, &states_d, &trans_seg, &trans_dense[0], &trans_dense[1], &seg_counts,
                      &seg_status, &seam_ptrs, &mismatch_d, &run_counts, &run_offsets, &scan_scr, &maps_d,
                      &prefix_d, &cnts_d, &cprefix_d, &line_scr, &ctx_d, &events_d[0], &events_d[1], &sym_d[0], &sym_d[1], &bits0_d[0],
                      &bits0_d[1], &bits1_d[0], &bits1_d[1], &em_d[0], &em_d[1], &fx_d[0], &fx_d[1],
@@ -596,6 +600,7 @@ int Stream::finish_warmup() {
 
 int64_t Stream::push(const void *items, int64_t n, int mem, int *called_back) {
     if (called_back) *called_back = 0;
+    batch_fill.clear();  // the slicer writes the class bitmap at this stream's positions
     if (n < 0) {
         set_error("negative item count");
         return -1;
@@ -686,15 +691,16 @@ int64_t Stream::push(const void *items, int64_t n, int mem, int *called_back) {
 
 // A batch of independent captures in one pass (BASELINE.json configs[3]).  The reference gives every capture its own
 // transition_sink (own warm-up, own lo_val / hi_val: transition_sink.py:12-34,109-125), background thread, decoders and
-// PacketProcessors (decoder.py:29-33).  Here capture c owns the stream positions [c * pitch, c * pitch + cap_len) of one
-// position space (pitch: cap_len rounded up to tiles); one launch of the streaming slicer runs one segment per capture
-// from the capture's own warm-up state (computed on the device), and extraction / runs / line code walk the batch as one
-// stream in which a capture's first event finds decoders and PacketProcessors as new (linecode.cu).  Frames come out with
-// positions of that space: capture = pos / pitch, index in the capture = pos % pitch.
+// PacketProcessors (decoder.py:29-33).  Here capture c owns the positions [starts[c], starts[c + 1]) of one position space
+// (its length rounded up to tiles; nothing for a capture of at most av_window items, which the warm-up consumes whole); one
+// launch of the streaming slicer runs one segment per capture from the capture's own warm-up state (computed on the
+// device), and extraction / runs / line code walk the batch as one stream in which a capture's first event finds decoders
+// and PacketProcessors as new (linecode.cu, through a device table of the captures' starts and lengths).  Frames come out
+// with positions of that space: the capture is the last c with starts[c] <= pos, the index in it pos - starts[c].
 // Returns n_cap, -1 on error, -3 when a capture leaves the exactly-summable regime (the caller decodes captures one by
 // one then: nfc_stream_push takes the sequential path for such input).
-int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t cap_len, int64_t stride_items, const double *lo_vals,
-                           const double *hi_vals, int64_t *pitch_out) {
+int64_t Stream::push_batch_ragged(const void *const *items, int mem, int64_t n_cap, const int64_t *lengths, const double *lo_vals,
+                                  const double *hi_vals, int64_t *starts_out) {
     NFC_CUDA_CHECK(cudaSetDevice(prm.device));
     const int L = sp.L;
     const int T = tile();
@@ -707,32 +713,78 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
         set_error("push_batch: needs the streaming slicer (av_window in [1024, 52000], a multiple of 4)");
         return -1;
     }
-    if (n_cap <= 0 || cap_len <= (int64_t)L + 2 * sp.mx || stride_items < cap_len || L <= sp.mx + 1) {
-        set_error("push_batch: bad shape (captures %lld, items %lld, stride %lld, av_window %d)", (long long)n_cap, (long long)cap_len,
-                  (long long)stride_items, L);
+    // Any capture longer than L items is decoded on the device, however short its own range [L, length) is; there is no
+    // bound of L + 2 max_len.  Its segment starts from the exact state of its warm-up (batch_warm_kernel), not from a
+    // speculative start, so no seam, checkpoint or halo needs a minimum length.  Behind it lie val == 0 positions (padding,
+    // then the next capture's warm-up of L > max_len + 1 samples), so every run open at its end times out and resets
+    // cur_state (transition_sink.py:95-99) before the next capture's first own sample; the events at or past its length
+    // are not the capture's and the line code ignores them.  L > max_len + 1 is what that needs.
+    if (n_cap <= 0 || n_cap >= ((int64_t)1 << 31) || L <= sp.mx + 1) {
+        set_error("push_batch: bad shape (captures %lld, av_window %d, max_len %d)", (long long)n_cap, L, sp.mx);
         return -1;
     }
     if (prm.outputs & NFC_OUT_DROPPED_EVENTS) {
         set_error("push_batch: type -1 events are not reproduced across capture boundaries (NFC_OUT_DROPPED_EVENTS)");
         return -1;
     }
-    if (((size_t)stride_items * ib) % 16 != 0 || ((uintptr_t)items % 16) != 0) {
-        set_error("push_batch: captures must start 16-byte aligned");
-        return -1;
+    // ---- layout: starts[c + 1] = starts[c] + the capture's length rounded up to tiles (0 for at most L items)
+    std::vector<int64_t> starts((size_t)n_cap + 1, 0);
+    for (int64_t c = 0; c < n_cap; c++) {
+        const int64_t len = lengths[c];
+        if (len < 0 || (len > 0 && !items[c])) {
+            set_error("push_batch: capture %lld: bad length %lld or null items", (long long)c, (long long)len);
+            return -1;
+        }
+        const int64_t width = len > L ? (len + T - 1) / T * T : 0;
+        if (width >= ((int64_t)1 << 30)) {
+            set_error("push_batch: capture %lld too long for one slab (%lld items): decode it with nfc_stream_push", (long long)c,
+                      (long long)len);
+            return -1;
+        }
+        if (width && mem == NFC_MEM_DEVICE && ((uintptr_t)items[c] % 16) != 0) {
+            set_error("push_batch: capture %lld: device items must start 16-byte aligned", (long long)c);
+            return -1;
+        }
+        starts[(size_t)c + 1] = starts[(size_t)c] + width;
     }
-    const int64_t pitch = (cap_len + T - 1) / T * T;
-    if (pitch >= ((int64_t)1 << 30)) {
-        set_error("push_batch: capture too long for one slab");
-        return -1;
-    }
-    if (pitch_out) *pitch_out = pitch;
-    const void *d_items = items;
+    if (starts_out) memcpy(starts_out, starts.data(), sizeof(int64_t) * ((size_t)n_cap + 1));
+    // ---- the captures' items on the device; host captures are staged into 16-byte aligned slots, one copy per run of
+    // captures that lie exactly one behind the other in host memory (a contiguous 2-D batch is one copy).  Nothing between
+    // two captures is read: that memory is not the caller's to give, and may not even be mapped.
+    std::vector<const void *> d_in((size_t)n_cap, nullptr);
     if (mem == NFC_MEM_HOST) {
-        const size_t bytes = ((size_t)(n_cap - 1) * (size_t)stride_items + (size_t)cap_len) * ib;
-        if (batch_stage.ensure(bytes + 64)) return -1;
-        NFC_CUDA_CHECK(cudaMemcpyAsync(batch_stage.p, items, bytes, cudaMemcpyHostToDevice, cs));
-        stats.h2d_bytes += (int64_t)bytes;
-        d_items = batch_stage.p;
+        struct Run { const char *h; size_t bytes, slot; };
+        std::vector<Run> runs;
+        std::vector<std::pair<size_t, size_t>> where((size_t)n_cap);  // (run, byte offset in it)
+        size_t total_bytes = 0;
+        const char *prev = nullptr;
+        size_t prev_bytes = 0;
+        for (int64_t c = 0; c < n_cap; c++) {
+            if (starts[(size_t)c + 1] == starts[(size_t)c]) continue;  // no segment: its items are not read
+            const char *h = (const char *)items[c];
+            const size_t bytes = (size_t)lengths[c] * ib;
+            const bool joins = prev && h == prev + prev_bytes && (size_t)(h - runs.back().h) % 16 == 0;
+            if (!joins) {
+                total_bytes = (total_bytes + 255) / 256 * 256;
+                runs.push_back(Run{h, 0, total_bytes});
+            }
+            Run &r = runs.back();
+            where[(size_t)c] = {runs.size() - 1, (size_t)(h - r.h)};
+            const size_t end = (size_t)(h - r.h) + bytes;
+            total_bytes += end - r.bytes;
+            r.bytes = end;
+            prev = h;
+            prev_bytes = bytes;
+        }
+        if (batch_stage.ensure(total_bytes + 64)) return -1;
+        for (const Run &r : runs) {
+            NFC_CUDA_CHECK(cudaMemcpyAsync(batch_stage.as<char>() + r.slot, r.h, r.bytes, cudaMemcpyHostToDevice, cs));
+            stats.h2d_bytes += (int64_t)r.bytes;
+        }
+        for (int64_t c = 0; c < n_cap; c++)
+            if (starts[(size_t)c + 1] != starts[(size_t)c]) d_in[(size_t)c] = batch_stage.as<char>() + runs[where[(size_t)c].first].slot + where[(size_t)c].second;
+    } else {
+        for (int64_t c = 0; c < n_cap; c++) d_in[(size_t)c] = items[c];
     }
     // ---- per-capture parameters (transition_sink's lo_val / hi_val constructor arguments)
     std::vector<SlicerParams> ps((size_t)n_cap, sp);
@@ -751,45 +803,56 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
     }
     if (params_d.ensure(sizeof(SlicerParams) * (size_t)n_cap)) return -1;
     NFC_CUDA_CHECK(cudaMemcpyAsync(params_d.p, ps.data(), sizeof(SlicerParams) * (size_t)n_cap, cudaMemcpyHostToDevice, cs));
-    // ---- warm-up states, bitmap, one segment per capture
+    // ---- the capture table of the line code: starts, then lengths (read by chains until the last slab is finalized)
+    std::vector<int64_t> tab(starts);
+    tab.insert(tab.end(), lengths, lengths + n_cap);
+    if (batch_tab.ensure(sizeof(int64_t) * tab.size())) return -1;
+    NFC_CUDA_CHECK(cudaMemcpyAsync(batch_tab.p, tab.data(), sizeof(int64_t) * tab.size(), cudaMemcpyHostToDevice, cs));
+    // ---- bitmap, one segment per capture, warm-up states
     const size_t sblk = state_block_bytes(L);
     if (batch_states.ensure(sblk * (size_t)n_cap) || seg_status.ensure(sizeof(int32_t) * (size_t)n_cap) ||
         works_d.ensure(sizeof(SegWork) * (size_t)n_cap))
         return -1;
-    const int64_t total = n_cap * pitch;
+    const int64_t total = starts[(size_t)n_cap];
     const size_t n_chunks = (size_t)(total / 128);
+    std::vector<int64_t> fill;  // the segment ranges, in capture order
+    for (int64_t c = 0; c < n_cap; c++)
+        if (starts[(size_t)c + 1] != starts[(size_t)c]) {
+            fill.push_back(starts[(size_t)c] + L);
+            fill.push_back(starts[(size_t)c] + lengths[c]);
+        }
     const size_t bm_cap_before = bitmap_d.cap;
     if (bitmap_d.ensure((n_chunks + 64) * 32)) return -1;
-    if (bitmap_d.cap != bm_cap_before || batch_fill_pitch != pitch || batch_fill_caps < n_cap || batch_fill_len != cap_len) {
+    if (bitmap_d.cap != bm_cap_before || batch_fill.size() < fill.size() || batch_fill.empty() ||
+        !std::equal(fill.begin(), fill.end(), batch_fill.begin())) {
         if (launch_bitmap_fill(bitmap_d.as<uint32_t>(), n_chunks, cs)) return -1;
-        batch_fill_pitch = pitch;
-        batch_fill_caps = n_cap;
-        batch_fill_len = cap_len;
+        batch_fill = fill;
         stats.launches++;
     }
-    if (launch_batch_warm(d_items, (int64_t)((size_t)stride_items * ib), pitch, (int)n_cap, L, params_d.as<SlicerParams>(), batch_states.p,
-                          sblk, cs))
-        return -1;
-    stats.launches++;
-    // Captures take different times (the closer hi_val lies to the tag's HIGH level, the more of a capture's tiles need the
-    // precise passes) and there are more of them than CTAs fit on the device at once: the ones expected to take longest go
-    // first, so that the last wave is made of short ones.
-    std::vector<int64_t> order((size_t)n_cap);
-    for (int64_t c = 0; c < n_cap; c++) order[(size_t)c] = c;
-    if (hi_vals) std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return hi_vals[a] > hi_vals[b]; });
-    std::vector<SegWork> works((size_t)n_cap);
-    for (int64_t k = 0; k < n_cap; k++) {
+    // Captures take different times: the longer a capture, and the closer hi_val lies to the tag's HIGH level (the more of
+    // its tiles need the precise passes), the longer its segment runs.  There are more segments than CTAs fit on the device
+    // at once: the ones expected to take longest go first, so that the last wave is made of short ones.
+    std::vector<int64_t> order;
+    for (int64_t c = 0; c < n_cap; c++)
+        if (starts[(size_t)c + 1] != starts[(size_t)c]) order.push_back(c);
+    std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) {
+        if (lengths[a] != lengths[b]) return lengths[a] > lengths[b];
+        return hi_vals && hi_vals[a] > hi_vals[b];
+    });
+    const int n_works = (int)order.size();
+    std::vector<SegWork> works((size_t)n_works);
+    for (int k = 0; k < n_works; k++) {
         const int64_t c = order[(size_t)k];
         SegWork &w = works[(size_t)k];
         memset(&w, 0, sizeof(w));
-        const int64_t B = c * pitch;
-        w.in = (const char *)d_items + (size_t)c * (size_t)stride_items * ib;
+        const int64_t B = starts[(size_t)c];
+        w.in = d_in[(size_t)c];
         w.in_pos0 = B;
         w.in_begin = B;
-        w.in_end = B + cap_len;
+        w.in_end = B + lengths[c];
         w.warm_begin = B + L;
         w.begin = B + L;
-        w.end = B + cap_len;
+        w.end = B + lengths[c];
         w.slab_pos0 = 0;
         w.state_in = reinterpret_cast<const SlicerHdr *>(batch_states.as<char>() + sblk * (size_t)c);
         for (int j = 0; j < 3; j++) w.ckpt_pos[j] = INT64_MAX;
@@ -798,16 +861,20 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
         w.bitmap = bitmap_d.as<uint32_t>();
         w.bm_pos0 = 0;
     }
-    NFC_CUDA_CHECK(cudaMemcpyAsync(works_d.p, works.data(), sizeof(SegWork) * (size_t)n_cap, cudaMemcpyHostToDevice, cs));
-    if (launch_streaming(works_d.as<SegWork>(), (int)n_cap)) return -1;
-    stats.launches++;
-    stats.slicer_launches++;
-    stats.segments += n_cap;
-    std::vector<int32_t> status((size_t)n_cap);
-    NFC_CUDA_CHECK(cudaMemcpyAsync(status.data(), seg_status.p, sizeof(int32_t) * (size_t)n_cap, cudaMemcpyDeviceToHost, cs));
+    std::vector<int32_t> status((size_t)n_cap, 0);
+    if (n_works) {
+        NFC_CUDA_CHECK(cudaMemcpyAsync(works_d.p, works.data(), sizeof(SegWork) * (size_t)n_works, cudaMemcpyHostToDevice, cs));
+        if (launch_batch_warm(works_d.as<SegWork>(), n_works, L, params_d.as<SlicerParams>(), cs)) return -1;
+        stats.launches++;
+        if (launch_streaming(works_d.as<SegWork>(), n_works)) return -1;
+        stats.launches++;
+        stats.slicer_launches++;
+        stats.segments += n_works;
+        NFC_CUDA_CHECK(cudaMemcpyAsync(status.data(), seg_status.p, sizeof(int32_t) * (size_t)n_cap, cudaMemcpyDeviceToHost, cs));
+    }
     NFC_CUDA_CHECK(sync_cs());
-    add_kernel_time();
-    for (int64_t c = 0; c < n_cap; c++)
+    if (n_works) add_kernel_time();
+    for (int64_t c : order)
         if (status[(size_t)c] & (SEG_INEXACT | SEG_NOT_SANE)) {
             set_error("push_batch: capture %lld is outside the exactly-summable regime: decode the captures one by one", (long long)c);
             return -3;
@@ -817,31 +884,57 @@ int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t ca
     bm_lo = 0;
     bm_hi = total;
     bm_origin = 0;
-    lt.batch_pitch = (uint32_t)pitch;
+    batch_starts = starts;
+    lt.batch_tab = batch_tab.as<int64_t>();
+    lt.batch_n = (uint32_t)n_cap;
     lt.batch_skip = (uint32_t)L;
-    lt.batch_len = (uint32_t)cap_len;
-    // slabs of whole captures (nfc_stream_set_tuning's slab_len shortens them: tests)
+    // slabs of whole captures, packed greedily up to slab_max positions; a wider capture is a slab of its own
+    // (nfc_stream_set_tuning's slab_len shortens them: tests; more, shorter slabs were slower: 10.5 against 9.6 ms)
     const int64_t slab_max = slab_len > 0 ? std::min<int64_t>(slab_len, (int64_t)1 << 30) : (int64_t)1 << 30;
-    const int64_t per_slab = std::max<int64_t>(1, slab_max / pitch);  // (more, shorter slabs were slower: 10.5 against 9.6 ms)
     int rc = 0;
-    if (finish_pending()) return -1;
+    if (finish_pending()) rc = -1;
     // What a slab's chain inherits from the slab before (run carry, decoder state, the val before its first sample) does
     // not matter: a capture's warm-up flushes it, and its first event finds decoders and PacketProcessors as new.  So the
     // chains of the batch's slabs are queued back to back like those of one stream.
     run_carry = RunCarry{0, 0, L % sp.mx, 0};
-    for (int64_t c0 = 0; c0 < n_cap && !rc; c0 += per_slab) {
-        const int64_t c1 = std::min(n_cap, c0 + per_slab);
-        if (process_slab(nullptr, c0 * pitch, c0 * pitch, c1 * pitch, c0 * pitch, c1 * pitch, c1 * pitch)) rc = -1;
-        pos = c1 * pitch;
-        stats.samples += (c1 - c0) * cap_len;
+    for (int64_t c0 = 0; c0 < n_cap && !rc;) {
+        int64_t c1 = c0 + 1;
+        while (c1 < n_cap && starts[(size_t)c1 + 1] - starts[(size_t)c0] <= slab_max) c1++;
+        const int64_t a = starts[(size_t)c0], b = starts[(size_t)c1];
+        if (b > a && process_slab(nullptr, a, a, b, a, b, b)) rc = -1;
+        pos = b;
+        for (int64_t c = c0; c < c1; c++) stats.samples += lengths[c];
+        c0 = c1;
     }
     if (!rc && finish_pending()) rc = -1;
-    lt.batch_pitch = 0;
+    lt.batch_tab = nullptr;
+    lt.batch_n = 0;
     bm_lo = bm_hi = 0;
     // the parameter block of a single stream again
     cudaMemcpyAsync(params_d.p, &sp, sizeof(sp), cudaMemcpyHostToDevice, cs);
     if (sync_cs() != cudaSuccess && !rc) rc = -1;
     return rc ? rc : n_cap;
+}
+
+// Equally long captures at items + c * stride_items: the ragged batch with starts[c] = c * pitch.
+int64_t Stream::push_batch(const void *items, int mem, int64_t n_cap, int64_t cap_len, int64_t stride_items, const double *lo_vals,
+                           const double *hi_vals, int64_t *pitch_out) {
+    const size_t ib = item_bytes(sp.input_kind);
+    if (n_cap <= 0 || cap_len <= (int64_t)sp.L || stride_items < cap_len) {
+        set_error("push_batch: bad shape (captures %lld, items %lld, stride %lld, av_window %d)", (long long)n_cap, (long long)cap_len,
+                  (long long)stride_items, sp.L);
+        return -1;
+    }
+    if (((size_t)stride_items * ib) % 16 != 0 || ((uintptr_t)items % 16) != 0) {
+        set_error("push_batch: captures must start 16-byte aligned");
+        return -1;
+    }
+    std::vector<const void *> ptrs((size_t)n_cap);
+    for (int64_t c = 0; c < n_cap; c++) ptrs[(size_t)c] = (const char *)items + (size_t)c * (size_t)stride_items * ib;
+    std::vector<int64_t> lengths((size_t)n_cap, cap_len), starts((size_t)n_cap + 1);
+    const int64_t rc = push_batch_ragged(ptrs.data(), mem, n_cap, lengths.data(), lo_vals, hi_vals, starts.data());
+    if (rc >= 0 && pitch_out) *pitch_out = starts[1];
+    return rc;
 }
 
 // Launches the streaming slicer kernel between ev_k0 and ev_k1; add_kernel_time() counts its time once the stream has been
@@ -1462,14 +1555,19 @@ int Stream::post_chain(int64_t a, int64_t b, bool from_bitmap, uint32_t R_host, 
     NFC_CUDA_CHECK(cudaStreamWaitEvent(csL, evR[ci], 0));
     if (ev_out_set[oi]) NFC_CUDA_CHECK(cudaStreamWaitEvent(csL, ev_out[oi], 0));  // the records of slab k-2 have left this output set
     j.have_line = want_line;
+    LineTables slt = lt;  // a batch's slab: its first capture and position (also when the slab is done again later)
+    if (slt.batch_tab) {
+        slt.batch_base = a;
+        slt.batch_c0 = (uint32_t)(std::lower_bound(batch_starts.begin(), batch_starts.end(), a) - batch_starts.begin());
+    }
     if (want_line) {
         const uint32_t nc = std::max(1u, linecode_chunks(j.cap_M));
         if (start_d.ensure((size_t)nc * 2 + 64) || summ_d.ensure((size_t)nc * 2 + 64) || cnts_d.ensure((size_t)nc * linecode_cnt_bytes()) ||
             cprefix_d.ensure((size_t)nc * linecode_cnt_bytes()) || line_scr.ensure(linecode_scratch_bytes(nc) + 256))
             return -1;
         const EventRec *ev = events_d[oi].as<EventRec>();
-        if (launch_linecode_start(ev, &cx->M, j.cap_M, lt, &cp->dc_out, summ_d.as<uint16_t>(), start_d.as<uint16_t>(), &cx->flags, csL)) return -1;
-        if (launch_linecode_count(ev, &cx->M, j.cap_M, lt, start_d.as<uint16_t>(), cnts_d.p, cprefix_d.p, line_scr.p, cx->tot, csL)) return -1;
+        if (launch_linecode_start(ev, &cx->M, j.cap_M, slt, &cp->dc_out, summ_d.as<uint16_t>(), start_d.as<uint16_t>(), &cx->flags, csL)) return -1;
+        if (launch_linecode_count(ev, &cx->M, j.cap_M, slt, start_d.as<uint16_t>(), cnts_d.p, cprefix_d.p, line_scr.p, cx->tot, csL)) return -1;
         stats.launches += 6;
         if (j.exact) {
             PostCtx hx;
@@ -1479,9 +1577,9 @@ int Stream::post_chain(int64_t a, int64_t b, bool from_bitmap, uint32_t R_host, 
                 // some chunk saw no decoder reset within the search limit: compose chunk transfer functions instead
                 stats.linecode_scan_fallbacks++;
                 if (maps_d.ensure((size_t)nc * linecode_map_bytes()) || prefix_d.ensure((size_t)nc * linecode_map_bytes())) return -1;
-                if (launch_linecode_start_scan(ev, &cx->M, j.cap_M, lt, &cp->dc_out, maps_d.p, prefix_d.p, line_scr.p, start_d.as<uint16_t>(), csL))
+                if (launch_linecode_start_scan(ev, &cx->M, j.cap_M, slt, &cp->dc_out, maps_d.p, prefix_d.p, line_scr.p, start_d.as<uint16_t>(), csL))
                     return -1;
-                if (launch_linecode_count(ev, &cx->M, j.cap_M, lt, start_d.as<uint16_t>(), cnts_d.p, cprefix_d.p, line_scr.p, cx->tot, csL)) return -1;
+                if (launch_linecode_count(ev, &cx->M, j.cap_M, slt, start_d.as<uint16_t>(), cnts_d.p, cprefix_d.p, line_scr.p, cx->tot, csL)) return -1;
                 stats.launches += 9;
                 NFC_CUDA_CHECK(cudaMemsetAsync(&cx->flags, 0, 4, csL));
                 NFC_CUDA_CHECK(cudaMemcpyAsync(&hx, cx, 64, cudaMemcpyDeviceToHost, csL));
@@ -1495,7 +1593,7 @@ int Stream::post_chain(int64_t a, int64_t b, bool from_bitmap, uint32_t R_host, 
             bits1_d[oi].ensure((size_t)j.cap_b1 + 16) || em_d[oi].ensure(((size_t)j.cap_em + 16) * linecode_emission_bytes()) ||
             fx_d[oi].ensure(((size_t)j.cap_em + 16) * 8))
             return -1;
-        if (launch_linecode_write(ev, &cx->M, j.cap_M, lt, start_d.as<uint16_t>(), cprefix_d.p, want_sym ? sym_d[oi].as<SymbolRec>() : nullptr,
+        if (launch_linecode_write(ev, &cx->M, j.cap_M, slt, start_d.as<uint16_t>(), cprefix_d.p, want_sym ? sym_d[oi].as<SymbolRec>() : nullptr,
                                   want_sym ? j.cap_sym : 0, bits0_d[oi].as<uint8_t>(), j.cap_b0, bits1_d[oi].as<uint8_t>(), j.cap_b1, em_d[oi].p,
                                   fx_d[oi].p, j.cap_em, a, cp->bits_out, cx->bits_out, &cx->n_empty, &cx->n_frames, cp->pend_out, &cp->dc_out, &cx->dc_out,
                                   cx->pend_out, csL))
@@ -1873,6 +1971,16 @@ int64_t nfc_stream_push_batch(nfc_stream *h, const void *items, int mem, int64_t
     }
     if (h->s.settle()) return -1;
     return h->s.push_batch(items, mem, n_captures, items_per_capture, stride_items, lo_vals, hi_vals, pitch);
+}
+
+int64_t nfc_stream_push_batch_ragged(nfc_stream *h, const void *const *items, int mem, int64_t n_captures, const int64_t *lengths,
+                                     const double *lo_vals, const double *hi_vals, int64_t *starts) {
+    if (!h || !items || !lengths || !starts) {
+        nfc::set_error("null argument");
+        return -1;
+    }
+    if (h->s.settle()) return -1;
+    return h->s.push_batch_ragged(items, mem, n_captures, lengths, lo_vals, hi_vals, starts);
 }
 
 int64_t nfc_stream_push_events(nfc_stream *h, const nfc_event *ev, int64_t n) {
